@@ -10,7 +10,7 @@ HDRS := $(wildcard $(SRC)/*.h $(SRC)/*.cuh) include/pir_b200.h
 
 WIRE := pir_b200/lib/libpirb_wire.so
 
-all: $(LIB) $(WIRE) oracle build/shim_test build/shim_host_test build/wire_test build/device_math_host_test build/ctmul_host_test build/shim_bench
+all: $(LIB) $(WIRE) oracle build/shim_test build/shim_host_test build/wire_test build/wire_fuzz_test build/device_math_host_test build/ctmul_host_test build/shim_bench
 
 $(OBJ)/%.o: $(SRC)/%.cu $(HDRS)
 	@mkdir -p $(OBJ)

@@ -45,6 +45,8 @@ WORKLOADS = {
 }
 DEFAULT_QUERIES_PER_GPU = {"cfg4": 8}
 DB_SEED = 2024
+DUMP_LIMIT_BYTES = 64 * 10 ** 6  # --dump-outputs, over all ranks
+DUMP_SEED = 7
 
 
 def workload_string(name, ql, world):
@@ -70,6 +72,21 @@ def synth_inputs(N, mods, dims, n_queries, seed):
     elts = [(N >> i) + 1 for i in range(N.bit_length() - 1)]
     keys = random_limbs(rng, mods, (len(elts), k, 2), N)                           # [n][k][2][k+1][N]
     return queries, elts, keys
+
+
+def dump_replies(out_dir, name, replies, limit_bytes):
+    """out_dir/<name>.npy, a file of at most limit_bytes: the uint64 reply limbs as float64, exact because every limb is
+    below its < 2^53 modulus.  When the whole array does not fit, a seeded sample of flat positions in increasing order,
+    the same for every run of that shape."""
+    if replies.size and int(replies.max()) >= 1 << 53:
+        raise SystemExit("--dump-outputs: reply limbs of 53 bits or more have no exact float64 form")
+    vals = replies.astype(np.float64)
+    n = (limit_bytes - 4096) // vals.itemsize  # 4 KiB kept for the .npy header (128 bytes for these shapes)
+    if vals.size > n:
+        pick = np.random.default_rng(DUMP_SEED).choice(vals.size, n, replace=False)
+        vals = vals.reshape(-1)[np.sort(pick)]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, name + ".npy"), vals)
 
 
 class ClockSampler:
@@ -185,15 +202,11 @@ def run_reference(args):
 
     pool = ThreadPoolExecutor(cores)
     t_one = one(0)
-    steps = args.steps
-    # bound the whole run to a few minutes (a step = `cores` concurrent queries, one per thread)
-    t_step_guess = t_one * (1.0 if not sampled else 1.0) * 1.5
-    while steps > 1 and (steps + min(args.warmup, 1)) * t_step_guess > 200:
-        steps -= 1
-    for _ in range(min(args.warmup, 1)):
+    # a step = `cores` concurrent queries, one per thread
+    for _ in range(args.warmup):
         list(pool.map(one, range(cores)))
     est, wall = [], []
-    for _ in range(steps):
+    for _ in range(args.steps):
         s0 = time.perf_counter()
         est.extend(pool.map(one, range(cores)))
         wall.append(time.perf_counter() - s0)
@@ -205,7 +218,7 @@ def run_reference(args):
     qps = cores / step_s
     line = {
         "impl": "reference", "metric": "pir_queries_per_sec", "value": qps, "unit": "queries/s",
-        "n_gpus": args.gpus, "steps": steps, "warmup": min(args.warmup, 1), "ms_per_step": 1e3 * step_s,
+        "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup, "ms_per_step": 1e3 * step_s,
         "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "u64", "data": "synthetic",
         "config": {"workload": workload_string(args.workload, ql, max(1, args.gpus)), "queries_per_step": cores,
                    "num_pt": num_pt, "dims": dims},
@@ -303,9 +316,9 @@ def run_ours(args):
     qps = world * ql * args.steps / (total_ms / 1e3)
     reply_dev = out.clone()
 
-    # per-stage device times (CUDA events recorded by the library on its launching stream), measured live on a few
+    # per-stage device times (CUDA events recorded by the library on its launching stream), measured live on
     # extra steps: profiling inserts events between kernels, so those steps run eagerly instead of as one graph
-    stage_mean = srv.profile_stages(step_dev, flush_l2, min(args.steps, 10))
+    stage_mean = srv.profile_stages(step_dev, flush_l2, args.steps)
 
     # ---------------- roofline: the single-query database scan on this GPU's rows, timed live ----------------
     dimL = dims[-1] if d > 1 else None
@@ -315,7 +328,7 @@ def run_ours(args):
         sv1 = sharded.to_device(random_limbs(rng, mods[:k], (1, dimL, 2), N), dev)
         srv.set_profiling(True)
         ts = []
-        for i in range(3 + 7):
+        for i in range(3 + args.steps):
             flush_l2()
             srv.scan(sv1, want_rows=False)
             torch.cuda.synchronize()
@@ -357,6 +370,10 @@ def run_ours(args):
         dist.all_reduce(e2e_total, op=dist.ReduceOp.MAX)
     e2e_qps = world * ql * args.steps / float(e2e_total.item())
     e2e_same = bool(np.array_equal(out_np, sharded.to_host(reply_dev)))
+    if args.dump_outputs:
+        # the replies of the last timed step, [queries of this rank][reply_cts][2][k][N], as the caller receives them
+        dump_replies(args.dump_outputs, "replies" if world == 1 else "replies_rank%d" % rank,
+                     sharded.to_host(reply_dev), DUMP_LIMIT_BYTES // world)
 
     # ---------------- parity: the timed path against the CPU oracle (and, sharded, against the unsharded GPU path) ---
     parity, parity_detail, cpu = None, None, None
@@ -411,12 +428,12 @@ def run_ours(args):
     # ---------------- N=1: the C++ drop-in itself (pir::PIRServer::ProcessRequest of the shim), limbs and wire bytes ----
     shim = None
     if world == 1 and not args.no_shim:
-        shim = run_shim_bench(items, size, d, n, bits, ql, min(args.steps, 20))
+        shim = run_shim_bench(items, size, d, n, bits, ql, args.steps)
 
     # ---------------- N=1: single-query latency on BASELINE configs[1] ----------------
     latency_cfg2 = None
     if world == 1 and args.workload != "cfg2" and not args.no_cfg2:
-        latency_cfg2 = cfg2_latency(pb, sharded, torch, dev, local_rank, flush_l2)
+        latency_cfg2 = cfg2_latency(pb, sharded, torch, dev, local_rank, flush_l2, args.steps)
 
     if rank != 0:
         if world > 1:
@@ -439,8 +456,9 @@ def run_ours(args):
         roofline = {"kernel": "k_scan", "bound": "hbm", "achieved": achieved, "peak": peak, "unit": "GB/s",
                     "frac": achieved / peak, "traffic": traffic, "traffic_source": traffic_src if traffic else None,
                     "peak_source": peak_src, "bytes_per_launch": scan_bytes, "ms_per_launch": scan_ms,
-                    "what": "single-query scan of this GPU's rows of the database (%d plaintexts), 7 launches after 3 "
-                            "warm-ups, CUDA events on the launching stream, L2 flushed between launches" % srv.pt_count}
+                    "what": "single-query scan of this GPU's rows of the database (%d plaintexts), %d launches after 3 "
+                            "warm-ups, CUDA events on the launching stream, L2 flushed between launches" % (
+                                srv.pt_count, args.steps)}
 
     # ---------------- expansion (FP64-pipe-bound): algorithmic FP64 operations of the key switches / stage time -----
     # per key switch: k(k+1) forward + 2(k+1) inverse transforms of N/2*log2(N) butterflies at 8 FP64 ops, 2k(k+1)N
@@ -511,7 +529,7 @@ def run_shim_bench(items, size, d, n, bits, nq, steps, n_gpus=1):
         return {"e2e_cpp": {"unavailable": "%s: %s" % (type(e).__name__, e)}, "e2e_wire": None}
 
 
-def cfg2_latency(pb, sharded, torch, dev, local_rank, flush_l2, steps=30):
+def cfg2_latency(pb, sharded, torch, dev, local_rank, flush_l2, steps):
     """Single-query latency on BASELINE configs[1] (d=2, 2^16 x 288 B): device-resident and through ProcessRequest."""
     items, size, d, n, bits, desc = WORKLOADS["cfg2"]
     params = pb.CreatePIRParameters(items, size, d, pb.GenerateEncryptionParams(n, bits))
@@ -536,7 +554,7 @@ def cfg2_latency(pb, sharded, torch, dev, local_rank, flush_l2, steps=30):
         ev[i][1].record()
     torch.cuda.synchronize()
     ms = [a.elapsed_time(b) for a, b in ev]
-    stages = srv.profile_stages(lambda: srv.answer(d_q), flush_l2, 10)
+    stages = srv.profile_stages(lambda: srv.answer(d_q), flush_l2, steps)
     q_pin = torch.from_numpy(queries.view(np.int64)).pin_memory()
     out_pin = torch.empty((1, srv.ctx.reply_cts, 2, k, N), dtype=torch.int64).pin_memory()
     server = pb.PIRServer(srv.db, params)
@@ -557,8 +575,13 @@ def cfg2_latency(pb, sharded, torch, dev, local_rank, flush_l2, steps=30):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
-    ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--steps", type=int, default=20,
+                    help="timed steps of every timed loop: the headline device loop, the end-to-end loop, the per-stage "
+                         "profile, the k_scan roofline launches, the C++ shim bench, the cfg2 latency and the reference "
+                         "arm; only the single-thread CPU baseline keeps its own bound (up to 5 oracle queries or 12 s)")
+    ap.add_argument("--warmup", type=int, default=3,
+                    help="untimed steps before the headline loop (the GPU arm runs at least 3: the second call of a "
+                         "shape captures its CUDA graph, the third replays it)")
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="cfg4", choices=sorted(WORKLOADS))
     ap.add_argument("--queries-per-gpu", type=int, default=None)
@@ -571,7 +594,15 @@ def main():
                          "(default) or by NCCL all-gather")
     ap.add_argument("--scan-traffic", type=float, default=None,
                     help="dram bytes per scan launch; default: the committed ncu capture in profiles/ for this workload")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the replies of the last one to DIR/replies.npy (with --gpus > 1, "
+                         "DIR/replies_rank<r>.npy per rank) as exact float64, at most 64 MB in all; the inputs are seeded, "
+                         "so two builds run with the same arguments can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the replies of the GPU path; --impl reference has none")
     if args.queries_per_gpu is None:
         args.queries_per_gpu = DEFAULT_QUERIES_PER_GPU.get(args.workload, 1)
     if args.gpus > 1 and "WORLD_SIZE" not in os.environ:
