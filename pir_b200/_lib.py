@@ -74,14 +74,6 @@ SYMBOLS = {
     "pirb_multiply_partial_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p]),
     "pirb_reduce_finish_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint64, C.c_uint32, C.c_void_p,
                                          C.c_void_p]),
-    "pirb_reduce_finish_peers_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32, C.c_void_p,
-                                               C.c_void_p]),
-    "pirb_xbuf_create": (C.c_int, [C.c_void_p, C.c_uint32, C.c_uint32, C.c_void_p]),
-    "pirb_xbuf_open": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32]),
-    "pirb_answer_partial_xbuf_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint64, C.c_uint32,
-                                               C.c_void_p]),
-    "pirb_multiply_partial_xbuf_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32, C.c_void_p]),
-    "pirb_reduce_finish_xbuf_dev": (C.c_int, [C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.c_void_p, C.c_void_p]),
     "pirb_dist_create": (C.c_int, [C.c_void_p, C.c_uint32, C.c_uint32, C.c_void_p, C.POINTER(C.c_void_p)]),
     "pirb_dist_open_ipc": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32]),
     "pirb_dist_attach": (C.c_int, [C.c_void_p, C.POINTER(C.c_void_p), C.c_uint32, C.c_uint32]),

@@ -145,13 +145,6 @@ struct pirb_ctx {
   struct GraphEntry { cudaGraphExec_t exec = nullptr; unsigned long long epoch = 0; u64 launches = 0; };
   std::map<std::tuple<int, u32, unsigned long long, const void*, const void*>, GraphEntry> graphs;  // (op, Q, key id, in, out)
   bool use_graphs = true;
-  // peer-memory exchange of partial replies (CUDA IPC over NVLink): own slots + the peers' mapped base pointers
-  u64* xbuf = nullptr;
-  u64 xslot_limbs = 0;
-  u32 xslots = 0;
-  std::vector<void*> xpeer_open;  // mappings to close
-  DevBuf xptrs;                   // device table [n_ranks] of base pointers (own + peers)
-  u32 xranks = 0;
   // Multi-GPU exchange over NVLink peer memory (pirb_dist_*): one block per rank that every peer maps:
   //   [ flags: err | sv[n_sub][n_ranks] | part[n_sub][n_ranks] ] [ sv slot 0 | sv slot 1 ] [ partial slot 0 | slot 1 ]
   struct Dist {
@@ -170,7 +163,6 @@ struct pirb_ctx {
     u64 flag_limbs = 0, sv_slot_limbs = 0, part_slot_limbs = 0;
     u64* base = nullptr;
     size_t bytes = 0;
-    std::vector<u64*> peer_base;
     std::vector<void*> opened;                // IPC mappings to close
     DevBuf peer_table;
     DevBuf self_table;                        // every entry = own block: the solo warm-up step exchanges with itself
@@ -215,8 +207,8 @@ struct pirb_ctx {
     u64 work_bytes = 4ull << 30;  // products of a level are formed for as many queries at a time as fit this budget
   } ct;
   pirb_ctx() {
-    for (DevBuf* b : {&db, &stage, &work, &dig, &acc, &xch, &part, &bufA[0], &bufA[1], &pts, &qbuf, &rbuf, &svbuf, &xptrs,
-                      &dbg, &dist.peer_table, &dist.self_table, &dist.stage, &tc.dbT, &tc.svT})
+    for (DevBuf* b : {&db, &stage, &work, &dig, &acc, &xch, &part, &bufA[0], &bufA[1], &pts, &qbuf, &rbuf, &svbuf, &dbg,
+                      &dist.peer_table, &dist.self_table, &dist.stage, &tc.dbT, &tc.svT})
       b->epoch = &alloc_epoch;
   }
 };
@@ -1041,7 +1033,6 @@ void pirb_ctx_destroy(pirb_ctx* c) {
   for (auto& kv : c->graphs)
     if (kv.second.exec) cudaGraphExecDestroy(kv.second.exec);
   if (c->tc.err) cudaFreeHost(c->tc.err);
-  for (void* pm : c->xpeer_open) cudaIpcCloseMemHandle(pm);
   {
     pirb_ctx::Dist& D = c->dist;
     for (void* pm : D.opened) cudaIpcCloseMemHandle(pm);
@@ -1056,7 +1047,6 @@ void pirb_ctx_destroy(pirb_ctx* c) {
     for (cudaEvent_t e_ : D.xprof)
       if (e_) cudaEventDestroy(e_);
   }
-  if (c->xbuf) cudaFree(c->xbuf);
   if (c->stream) cudaStreamDestroy(c->stream);
   if (c->side) cudaStreamDestroy(c->side);
   if (c->ev_fork) cudaEventDestroy(c->ev_fork);
@@ -1484,88 +1474,6 @@ int pirb_reduce_finish_dev(pirb_ctx* c, const uint64_t* d_partials, uint32_t n_p
   return 0;
 }
 
-int pirb_reduce_finish_peers_dev(pirb_ctx* c, const uint64_t* const* d_peer_ptrs, uint32_t n_parts,
-                                 uint32_t n_queries, uint64_t* d_replies, void* stream) {
-  if (!c || !d_peer_ptrs || !d_replies || !n_parts) return fail(PIRB_INVALID_ARGUMENT, "bad argument");
-  CU(cudaSetDevice(c->device));
-  cudaStream_t st = stream ? (cudaStream_t)stream : c->stream;
-  const u64 cts = (u64)n_queries * c->reply_cts;
-  RC(c->rbuf.ensure(cts * c->ctL * sizeof(u64)));
-  DevCallOrder order(c, st);
-  LAUNCH(c, launch_modadd_reduce_ptrs(c->P, reinterpret_cast<const u64* const*>(d_peer_ptrs), (int)n_parts, 0, c->rbuf.p, cts, st));
-  LAUNCH(c, launch_ntt_inv(c->P, c->rbuf.p, U(d_replies), (int)(cts * 2 * c->k), c->k, 0, 1, 0, 1, 0, 0, st));
-  return 0;
-}
-
-// ---- peer-memory exchange (SURVEY §8e: "direct P2P loads in the reduce kernel") ------------------------------------
-int pirb_xbuf_create(pirb_ctx* c, uint32_t max_queries, uint32_t n_slots, uint8_t* handle_out) {
-  if (!c || !handle_out || !max_queries || !n_slots) return fail(PIRB_INVALID_ARGUMENT, "bad argument");
-  CU(cudaSetDevice(c->device));
-  if (c->xbuf) return fail(PIRB_INVALID_ARGUMENT, "exchange buffer already created");
-  c->xslot_limbs = (u64)max_queries * c->reply_cts * c->ctL;
-  c->xslots = n_slots;
-  CU(cudaMalloc(&c->xbuf, c->xslot_limbs * n_slots * sizeof(u64)));
-  ++c->alloc_epoch;
-  cudaIpcMemHandle_t h;
-  CU(cudaIpcGetMemHandle(&h, c->xbuf));
-  static_assert(sizeof(h) == 64, "CUDA IPC handles are 64 bytes");
-  memcpy(handle_out, &h, 64);
-  return 0;
-}
-
-int pirb_xbuf_open(pirb_ctx* c, const uint8_t* handles, uint32_t n_ranks, uint32_t self_rank) {
-  if (!c || !handles || !c->xbuf || self_rank >= n_ranks) return fail(PIRB_INVALID_ARGUMENT, "bad argument");
-  CU(cudaSetDevice(c->device));
-  std::vector<u64*> table(n_ranks);
-  for (u32 r = 0; r < n_ranks; ++r) {
-    if (r == self_rank) { table[r] = c->xbuf; continue; }
-    cudaIpcMemHandle_t h;
-    memcpy(&h, handles + (size_t)r * 64, 64);
-    void* pm = nullptr;
-    CU(cudaIpcOpenMemHandle(&pm, h, cudaIpcMemLazyEnablePeerAccess));
-    c->xpeer_open.push_back(pm);
-    table[r] = (u64*)pm;
-  }
-  RC(c->xptrs.ensure(n_ranks * sizeof(u64*)));
-  CU(cudaMemcpy(c->xptrs.p, table.data(), n_ranks * sizeof(u64*), cudaMemcpyHostToDevice));
-  c->xranks = n_ranks;
-  return 0;
-}
-
-int pirb_multiply_partial_xbuf_dev(pirb_ctx* c, const uint64_t* d_sv_ntt, uint32_t n_queries, uint32_t slot,
-                                   void* stream) {
-  if (!c || !c->xbuf || slot >= c->xslots) return fail(PIRB_INVALID_ARGUMENT, "exchange buffer not set up");
-  if ((u64)n_queries * c->reply_cts * c->ctL > c->xslot_limbs) return fail(PIRB_INVALID_ARGUMENT, "too many queries for the slot");
-  return pirb_multiply_partial_dev(c, d_sv_ntt, n_queries, reinterpret_cast<uint64_t*>(c->xbuf + (u64)slot * c->xslot_limbs),
-                                   stream);
-}
-
-int pirb_answer_partial_xbuf_dev(pirb_ctx* c, const pirb_keys* keys, const uint64_t* d_queries, uint32_t n_queries,
-                                 uint64_t n_ct, uint32_t slot, void* stream) {
-  if (!c || !c->xbuf || slot >= c->xslots) return fail(PIRB_INVALID_ARGUMENT, "exchange buffer not set up");
-  if ((u64)n_queries * c->reply_cts * c->ctL > c->xslot_limbs) return fail(PIRB_INVALID_ARGUMENT, "too many queries for the slot");
-  return pirb_answer_partial_dev(c, keys, d_queries, n_queries, n_ct,
-                                 reinterpret_cast<uint64_t*>(c->xbuf + (u64)slot * c->xslot_limbs), stream);
-}
-
-// Caller guarantees (stream-ordered barrier, e.g. a tiny NCCL all-reduce) that every rank has finished writing `slot`.
-int pirb_reduce_finish_xbuf_dev(pirb_ctx* c, uint32_t slot, uint32_t q_first, uint32_t q_count, uint64_t* d_replies,
-                                void* stream) {
-  if (!c || !c->xbuf || !c->xranks || slot >= c->xslots || !d_replies) return fail(PIRB_INVALID_ARGUMENT, "exchange buffer not set up");
-  CU(cudaSetDevice(c->device));
-  cudaStream_t st = stream ? (cudaStream_t)stream : c->stream;
-  const u64 cts = (u64)q_count * c->reply_cts;
-  if (!cts) return 0;
-  RC(c->rbuf.ensure(cts * c->ctL * sizeof(u64)));
-  DevCallOrder order(c, st);
-  const u64 off = (u64)slot * c->xslot_limbs + (u64)q_first * c->reply_cts * c->ctL;
-  // the partial replies of every rank are loaded through the peer mappings inside the reducing kernel (NVLink P2P)
-  LAUNCH(c, launch_modadd_reduce_ptrs(c->P, reinterpret_cast<const u64* const*>(c->xptrs.p), (int)c->xranks, off, c->rbuf.p,
-                                      cts, st));
-  LAUNCH(c, launch_ntt_inv(c->P, c->rbuf.p, U(d_replies), (int)(cts * 2 * c->k), c->k, 0, 1, 0, 1, 0, 0, st));
-  return 0;
-}
-
 // ---- row-sharded serving with the exchange done by the kernels over NVLink peer memory (SURVEY §8e) ----------------
 // Per step and rank (all ranks run the same number of local queries in lockstep):
 //   producer stream  oblivious expansion of the rank's own queries: top levels for all of them at once, the wide
@@ -1666,7 +1574,6 @@ int pirb_dist_create(pirb_ctx* c, uint32_t max_local_queries, uint32_t sub_batch
 
 static int dist_finish_attach(pirb_ctx* c, const std::vector<u64*>& table) {
   pirb_ctx::Dist& D = c->dist;
-  D.peer_base = table;
   RC(D.peer_table.ensure(table.size() * sizeof(u64*)));
   CU(cudaMemcpy(D.peer_table.p, table.data(), table.size() * sizeof(u64*), cudaMemcpyHostToDevice));
   std::vector<u64*> self(table.size(), D.base);
@@ -1804,19 +1711,8 @@ static int dist_step(pirb_ctx* c, const pirb_keys* keys, const u64* d_queries, u
       if (xp) cudaEventRecord(D.xprof[3], D.xfer);
       const u64 row0 = (u64)D.rank * SB * 2 * D.g.nb;  // this rank's rows inside the sub-batch's region
       const u64 dst_off = (dist_sv_off(D, slot) + D.svt_off) * sizeof(u64) + sb * D.sub_bytes + row0 * D.g.Kp;
-      static const bool dma = getenv("PIRB_PUSH_DMA") && getenv("PIRB_PUSH_DMA")[0] == '1';
-      if (dma) {
-        // the same row push by the copy engines (one strided 2-D copy per rank): no SM is occupied by the transfer
-        if (!dry)
-          for (u32 r = 0; r < W; ++r) {
-            u8* dstp = reinterpret_cast<u8*>(solo ? D.base : D.peer_base[r]) + dst_off;
-            CU(cudaMemcpy2DAsync(dstp, (size_t)D.sub_rows * D.g.Kp, D.stage.p, (size_t)stage_rows * D.g.Kp,
-                                 (size_t)qn * 2 * D.g.nb * D.g.Kp, (size_t)c->k * c->N, cudaMemcpyDeviceToDevice, D.xfer));
-          }
-      } else {
-        LAUNCH(c, launch_push_rows(peers, W, reinterpret_cast<const u8*>(D.stage.p), (u64)stage_rows * D.g.Kp,
-                                   qn * 2 * D.g.nb * D.g.Kp, (u32)c->k * c->N, dst_off, (u64)D.sub_rows * D.g.Kp, D.xfer));
-      }
+      LAUNCH(c, launch_push_rows(peers, W, reinterpret_cast<const u8*>(D.stage.p), (u64)stage_rows * D.g.Kp,
+                                 qn * 2 * D.g.nb * D.g.Kp, (u32)c->k * c->N, dst_off, (u64)D.sub_rows * D.g.Kp, D.xfer));
       if (xp) cudaEventRecord(D.xprof[4], D.xfer);
     }
     LAUNCH(c, launch_signal(peers, W, dist_flag_off(D, 0, sb, D.rank), seq, D.xfer));

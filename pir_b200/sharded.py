@@ -1,20 +1,25 @@
 """Device-resident, row-sharded serving on top of the C ABI's *_dev entry points (SURVEY §8e).
 
-One process per GPU.  The database is split by rows of the first dimension; every rank expands the query
-(replicated, no communication), scans its rows, re-encodes and multiplies its share of the upper dimensions and
-produces a partial reply in NTT form.  The partials are combined with a mod-q add (never a plain integer sum):
-either NCCL all-gather + the fused add-and-inverse-NTT kernel, or peer pointers read directly over NVLink.
+One process per GPU.  The database is split by rows of the first dimension; every rank scans its rows for all ranks'
+queries, re-encodes and multiplies its share of the upper dimensions and produces partial replies in NTT form.  The
+partials are combined with a mod-q add (never a plain integer sum).  Two flows (setup_distributed picks one):
+- NVLink (d >= 2, when every rank can map its peers' memory; pirb_dist_*): the library's own kernels store the
+  selection vectors into the peers' memory and add the partial replies by peer loads;
+- NCCL (otherwise): the selection vectors (for d = 1 the query ciphertexts) and the partial replies are all-gathered
+  and every rank finishes its own queries with the fused add-and-inverse-NTT kernel.
 
 torch is used only for device memory, streams and torch.distributed — uint64 limbs are carried in int64 tensors.
 """
 import ctypes as C
-import os
 
 import numpy as np
 import torch
 
 from . import _lib
 from .api import GaloisKeys, PIRDatabase, PIRParameters, _check, _KeyHandle
+
+# Selection vectors of at least this many bytes per rank are exchanged split by ownership (_exchange_selection_vectors).
+SPLIT_EXCHANGE_MIN_BYTES = 64 << 20
 
 
 def _dp(t: torch.Tensor):
@@ -30,6 +35,7 @@ class ShardServer:
         self.ctx = self.db.ctx
         self.shard_index, self.shard_count = shard_index, shard_count
         self.keys = None
+        self._dist_mode = "nccl"
         with torch.cuda.device(self.device):
             self.stream = torch.cuda.Stream()
         self.k, self.N = self.ctx.k, self.ctx.N
@@ -127,26 +133,6 @@ class ShardServer:
         self._exit()
         return out
 
-    def reduce_finish_peers(self, peer_ptrs: torch.Tensor, n_queries: int) -> torch.Tensor:
-        """peer_ptrs: int64 cuda tensor of G device pointers (own + IPC-mapped peers) to partial buffers."""
-        out = self._empty(n_queries, self.ctx.reply_cts, 2, self.k, self.N)
-        st = self._enter()
-        _check(_lib.lib().pirb_reduce_finish_peers_dev(self.ctx.h, _dp(peer_ptrs), peer_ptrs.numel(), n_queries,
-                                                       _dp(out), st))
-        self._exit()
-        return out
-
-    def answer_distributed(self, d_queries: torch.Tensor) -> torch.Tensor:
-        """Row-sharded answer across the ranks of the default process group: partial -> all-gather -> mod-q add."""
-        import torch.distributed as dist
-        part = self.answer_partial(d_queries)
-        world = dist.get_world_size()
-        if world == 1:
-            return self.reduce_finish(part[None], d_queries.shape[0])
-        gathered = self._empty(world, *part.shape)
-        dist.all_gather_into_tensor(gathered, part)
-        return self.reduce_finish(gathered, d_queries.shape[0])
-
     def answer_batch_distributed(self, d_queries_local: torch.Tensor) -> torch.Tensor:
         """Batch path (SURVEY §8e): every rank expands only ITS queries, the NTT-form selection vectors are
         all-gathered, every rank multiplies ALL queries against its row shard, the partial replies are all-gathered
@@ -182,20 +168,6 @@ class ShardServer:
         self._exit()
         return out
 
-    # -- peer-memory exchange (CUDA IPC over NVLink) instead of the NCCL gather of partial replies ------------------
-    def setup_peer_exchange(self, max_queries: int, n_slots: int = 2):
-        """Collective: create this rank's exchange slots, swap IPC handles, map the peers' buffers."""
-        import torch.distributed as dist
-        world, rank = dist.get_world_size(), dist.get_rank()
-        handle = (C.c_uint8 * 64)()
-        _check(_lib.lib().pirb_xbuf_create(self.ctx.h, max_queries, n_slots, handle))
-        handles = [None] * world
-        dist.all_gather_object(handles, bytes(handle))
-        blob = (C.c_uint8 * (64 * world)).from_buffer_copy(b"".join(handles))
-        _check(_lib.lib().pirb_xbuf_open(self.ctx.h, blob, world, rank))
-        self._xslots, self._xslot = n_slots, 0
-        self._xflag = torch.zeros(1, dtype=torch.int32, device=self.device)
-
     def _gather_queries(self, d_queries_local: torch.Tensor) -> torch.Tensor:
         import torch.distributed as dist
         world = dist.get_world_size()
@@ -214,9 +186,7 @@ class ShardServer:
         sv_all = self._empty(world * ql, *sv_local.shape[1:])
         # measured on 8 B200s: at 10 MB per rank (config 2) the extra all-to-all costs more latency than the halved
         # volume saves, at 85-680 MB per rank (configs 3/4) the exchange is bandwidth-bound and the split wins.
-        # PIRB_SPLIT_EXCHANGE=1/0 forces the choice.
-        env = os.environ.get("PIRB_SPLIT_EXCHANGE")
-        split = env == "1" or (env is None and sv_local.numel() * 8 >= (64 << 20))
+        split = sv_local.numel() * 8 >= SPLIT_EXCHANGE_MIN_BYTES
         if world < 2 or len(self.params.dimensions) == 1 or not split:
             dist.all_gather_into_tensor(sv_all, sv_local)
             return sv_all
@@ -235,36 +205,13 @@ class ShardServer:
             sv_all[:, lo_me:hi_me] = recv.view(world * ql, hi_me - lo_me, *sv_local.shape[2:])
         return sv_all  # dimension-0 entries of other ranks' rows stay uninitialised: this shard never reads them
 
-    def answer_batch_distributed_p2p(self, d_queries_local: torch.Tensor) -> torch.Tensor:
-        """Like answer_batch_distributed, but the partial replies are not gathered: every rank writes them into its
-        own exchange slot and, after a stream-ordered barrier, each rank's reduce kernel loads all ranks' partials
-        for its own queries straight through the peer mappings (NVLink P2P) while adding them mod q."""
-        import torch.distributed as dist
-        world, rank = dist.get_world_size(), dist.get_rank()
-        ql = d_queries_local.shape[0]
-        if len(self.params.dimensions) == 1:
-            # one ciphertext of partial reply per query: nothing worth a peer-memory exchange (see the gather path)
-            return self.answer_batch_distributed(d_queries_local)
-        slot = self._xslot
-        sv_local = self.expand_ntt(d_queries_local)
-        sv_all = self._exchange_selection_vectors(sv_local)
-        st = self._enter()
-        _check(_lib.lib().pirb_multiply_partial_xbuf_dev(self.ctx.h, _dp(sv_all), world * ql, slot, st))
-        self._exit()
-        dist.all_reduce(self._xflag)  # barrier in stream order: every rank's slot is complete before anyone reads it
-        out = self._empty(ql, self.ctx.reply_cts, 2, self.k, self.N)
-        st = self._enter()
-        _check(_lib.lib().pirb_reduce_finish_xbuf_dev(self.ctx.h, slot, rank * ql, ql, _dp(out), st))
-        self._exit()
-        self._xslot = (slot + 1) % self._xslots
-        return out
-
     # -- one entry point for the multi-GPU step, whatever the transport ------------------------------------------
     def setup_distributed(self, queries_per_rank: int, prefer: str = "nvlink", sub_batch: int = 0) -> str:
         """Collective.  Chooses how selection vectors and partial replies travel between the ranks and sets it up;
         returns a description for the bench line.  "nvlink": the library's own kernels store / load peer memory
-        (pirb_dist_*; the process group is only used here, to swap the CUDA IPC handles).  Falls back to NCCL
-        collectives on every rank if any rank cannot map its peers' memory, and for one-dimensional databases."""
+        (pirb_dist_*; the process group is only used here, to swap the CUDA IPC handles).  Falls back to the NCCL flow
+        (answer_batch_distributed) on every rank if any rank cannot map its peers' memory, and for one-dimensional
+        databases; "nccl" always uses it."""
         import torch.distributed as dist
         world, rank = dist.get_world_size(), dist.get_rank()
         self._dist_mode = "nccl"
@@ -294,23 +241,11 @@ class ShardServer:
             if not ok:
                 import sys
                 sys.stderr.write("rank %d: peer-memory exchange unavailable (%s); using NCCL\n" % (rank, err))
-        if prefer != "nccl-gather" and len(self.params.dimensions) > 1:
-            try:
-                self.setup_peer_exchange(max_queries=world * queries_per_rank)
-                ok = 1
-            except Exception:  # noqa: BLE001
-                ok = 0
-            flag = torch.tensor([ok], device=self.device)
-            dist.all_reduce(flag, op=dist.ReduceOp.MIN)
-            if int(flag.item()):
-                self._dist_mode = "p2p"
-                return "selection vectors all-gathered with NCCL, partial replies reduced over NVLink peer loads"
         return "selection vectors and partial replies gathered with NCCL"
 
     def answer_dist(self, d_queries_local: torch.Tensor) -> torch.Tensor:
         """This rank's queries [ql][n_ct][2][k][N] -> this rank's replies; every rank calls it in lockstep."""
-        mode = getattr(self, "_dist_mode", "nccl")
-        if mode == "nvlink":
+        if self._dist_mode == "nvlink":
             ql, n_ct = d_queries_local.shape[0], d_queries_local.shape[1]
             out = self._empty(ql, self.ctx.reply_cts, 2, self.k, self.N)
             st = self._enter()
@@ -318,13 +253,11 @@ class ShardServer:
                                                    ql, n_ct, _dp(out), st))
             self._exit()
             return out
-        if mode == "p2p":
-            return self.answer_batch_distributed_p2p(d_queries_local)
         return self.answer_batch_distributed(d_queries_local)
 
     def answer_dist_host(self, q_pinned: torch.Tensor, out_pinned: torch.Tensor):
         """End-to-end variant: this rank's queries start in (pinned) host memory and its replies end there."""
-        if getattr(self, "_dist_mode", "nccl") == "nvlink":
+        if self._dist_mode == "nvlink":
             # the C ABI's host-buffer entry point: page-locked buffers are read / written in place by the kernels
             _check(_lib.lib().pirb_dist_answer(self.ctx.h, self.keys.h if self.keys else None,
                                                C.c_void_p(q_pinned.data_ptr()), q_pinned.shape[0], q_pinned.shape[1],
@@ -353,7 +286,7 @@ class ShardServer:
                     flush()
                 step()
                 torch.cuda.synchronize(self.device)
-                st = self.dist_stage_ms() if getattr(self, "_dist_mode", "") == "nvlink" else self.stage_ms()
+                st = self.dist_stage_ms() if self._dist_mode == "nvlink" else self.stage_ms()
                 for nm, v in st.items():
                     acc.setdefault(nm, []).append(v)
         finally:

@@ -1,4 +1,4 @@
-"""torchrun helper: row-sharded distributed answers must equal the unsharded answer (and the oracle) bit for bit.
+"""torchrun helper: row-sharded distributed answers must equal the oracle's answer on the whole database bit for bit.
 
 Run as: python -m torch.distributed.run --nproc-per-node N --master-addr 127.0.0.1 tests/helpers/dist_parity.py
 """
@@ -38,39 +38,32 @@ def main():
         srv.set_keys(gk)
         idxs = [(7 * r + 3) % dbsize for r in range(world)]
         queries = np.stack([cl.create_query(i) for i in idxs])          # [world][n_ct][2][k][N]
-        # (1) replicated expansion, every rank answers ALL queries
-        full = sharded.to_host(srv.answer_distributed(sharded.to_device(queries, dev)))
-        # (2) batch path: rank r expands only query r
+        db_ntt = oc.db_to_ntt(cl.orc, coeffs)
+        want = cl.orc.process_query(db_ntt, p.dimensions, cl.elts, cl.galois, queries[rank])
+        # (1) NCCL flow: rank r expands only query r
         mine = sharded.to_host(srv.answer_batch_distributed(sharded.to_device(queries[rank:rank + 1], dev)))[0]
-        ok &= bool(np.array_equal(full[rank], mine))
-        # (2b) the ownership-aware exchange of the selection vectors (chosen automatically for large messages)
-        os.environ["PIRB_SPLIT_EXCHANGE"] = "1"
+        ok &= bool(np.array_equal(mine, want))
+        # (1b) the ownership-aware exchange of the selection vectors (chosen automatically for large messages)
+        split_min, sharded.SPLIT_EXCHANGE_MIN_BYTES = sharded.SPLIT_EXCHANGE_MIN_BYTES, 0
         split = sharded.to_host(srv.answer_batch_distributed(sharded.to_device(queries[rank:rank + 1], dev)))[0]
-        del os.environ["PIRB_SPLIT_EXCHANGE"]
-        ok &= bool(np.array_equal(split, mine))
-        # (3) same, partial replies exchanged through peer memory (CUDA IPC) instead of an NCCL gather; run it three
-        #     times so both exchange slots and their reuse are exercised
-        srv.setup_peer_exchange(max_queries=world)
-        for _ in range(3):
-            p2p = sharded.to_host(srv.answer_batch_distributed_p2p(sharded.to_device(queries[rank:rank + 1], dev)))[0]
-            ok &= bool(np.array_equal(p2p, mine))
-        # (4) the exchange done by the library's own kernels over peer memory (pirb_dist_*, CUDA IPC between the
+        sharded.SPLIT_EXCHANGE_MIN_BYTES = split_min
+        ok &= bool(np.array_equal(split, want))
+        # (2) the exchange done by the library's own kernels over peer memory (pirb_dist_*, CUDA IPC between the
         #     processes): two local queries per rank in sub-batches of one, three steps
         if d >= 2:
+            nxt = (rank + 1) % world
+            want_nxt = cl.orc.process_query(db_ntt, p.dimensions, cl.elts, cl.galois, queries[nxt])
             mode = srv.setup_distributed(2, prefer="nvlink", sub_batch=1)
             ok &= srv._dist_mode == "nvlink"
-            two = np.stack([queries[rank], queries[(rank + 1) % world]])
+            two = np.stack([queries[rank], queries[nxt]])
             for _ in range(3):
                 nv = sharded.to_host(srv.answer_dist(sharded.to_device(two, dev)))
                 srv.dist_status()
-                ok &= bool(np.array_equal(nv[0], mine)) and bool(np.array_equal(nv[1], full[(rank + 1) % world]))
+                ok &= bool(np.array_equal(nv[0], want)) and bool(np.array_equal(nv[1], want_nxt))
             pin_q = torch.from_numpy(two.view(np.int64)).pin_memory()
             pin_r = torch.empty((2,) + nv.shape[1:], dtype=torch.int64).pin_memory()
             srv.answer_dist_host(pin_q, pin_r)                      # host-buffer entry point of the C ABI
             ok &= bool(np.array_equal(pin_r.numpy().view(np.uint64), nv))
-        # oracle on the whole database
-        want = cl.orc.process_query(oc.db_to_ntt(cl.orc, coeffs), p.dimensions, cl.elts, cl.galois, queries[rank])
-        ok &= bool(np.array_equal(mine, want))
         got = cl.process_response_strings([idxs[rank]], [mine])[0]
         ok &= got == items[idxs[rank]]
         if rank == 0:
