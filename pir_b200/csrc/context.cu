@@ -117,6 +117,11 @@ struct pirb_ctx {
     for (u64 i = first_local; i < first_local + n; ++i)
       if (!have[i]) { have[i] = 1; ++loaded; }
     tc.built = false;  // the byte-planar copy follows the database
+    // A captured answer graph scans the byte-planar copy as it was at capture time and never rebuilds it.  Drop them
+    // all: the next call of each shape runs eagerly (rebuilding the copy), the one after captures without the repack.
+    for (auto& kv : graphs)
+      if (kv.second.exec) cudaGraphExecDestroy(kv.second.exec);
+    graphs.clear();
   }
   u64 loaded_prefix() const {  // plaintexts loaded contiguously from the start of the shard
     if (loaded == pt_count) return pt_count;
@@ -355,9 +360,13 @@ int run_scan(pirb_ctx* c, const u64* sv_last, u64 sv_qstride, int n_queries, u32
   const DevParams& P = c->P;
   const u64 ctL = c->ctL;
   int n_split;
-  // small shards are launch-latency territory: the CUDA-core batched scan is as fast there
-  const bool use_tc = svt || (allow_tc && c->tc.min_queries > 0 && n_queries >= c->tc.min_queries &&
-                              npt >= c->tc.min_pt && tc_supported(P, dimL));
+  // small shards are launch-latency territory: the CUDA-core batched scan is as fast there; so is it for a last
+  // dimension too long for any tensor-core plan
+  TcPlan plan = {};
+  const bool want_tc = svt || (allow_tc && c->tc.min_queries > 0 && n_queries >= c->tc.min_queries && npt >= c->tc.min_pt);
+  const bool use_tc = want_tc && tc_launch_plan(P, dimL, (u32)n_queries, &plan);
+  // dist_layout chose the repacked exchange because a plan exists for the sub-batch, so one exists for these queries
+  if (svt && !use_tc) return fail(PIRB_INTERNAL, "tensor-core scan: no launch plan for the exchanged operand layout");
   if (use_tc) {
     // batch of queries: dense u8 contraction per coefficient slot on the tensor cores
     pirb_ctx::Tc& T = c->tc;
@@ -378,16 +387,15 @@ int run_scan(pirb_ctx* c, const u64* sv_last, u64 sv_qstride, int n_queries, u32
     c->scan_split = 1;
     RC(c->part.ensure((size_t)n_queries * n_rows * ctL * sizeof(u64)));
     if (svt) {
-      LAUNCH(c, launch_tc_scan_packed(P, T.g, reinterpret_cast<const u8*>(T.dbT.p), dimL, n_rows, svt->p, svt->rows_total,
+      LAUNCH(c, launch_tc_scan_packed(P, T.g, plan, reinterpret_cast<const u8*>(T.dbT.p), n_rows, svt->p, svt->rows_total,
                                       svt->row0, (u32)n_queries, T.err, c->sm_count, c->part.p, st));
     } else {
-      u32 qt, n_qt;
-      const u64 sv_bytes = tc_sv_bytes(P, T.g, (u32)n_queries, &qt, &n_qt);
+      const u64 sv_bytes = tc_sv_bytes(P, T.g, plan);
       if (sv_bytes > T.svT.bytes) {
         RC(T.svT.ensure(sv_bytes));
         CU(cudaMemsetAsync(T.svT.p, 0, sv_bytes, st));  // the K padding is never written afterwards
       }
-      LAUNCH(c, launch_tc_scan(P, T.g, reinterpret_cast<const u8*>(T.dbT.p), dimL, n_rows, sv_last, sv_qstride,
+      LAUNCH(c, launch_tc_scan(P, T.g, plan, reinterpret_cast<const u8*>(T.dbT.p), dimL, n_rows, sv_last, sv_qstride,
                                (u32)n_queries, reinterpret_cast<u8*>(T.svT.p), T.err, c->sm_count, c->part.p, st));
     }
   } else {
@@ -1497,11 +1505,14 @@ static int dist_layout(pirb_ctx* c, u32 max_local, u32 sub_q) {
   u64 mid = 0;
   for (int e = 1; e < c->d - 1; ++e) mid += c->dims[e];
   const u32 last = c->dims[c->d - 1];
-  // Tensor-core mode whenever the consumers' scans run on the tensor cores; the choice uses only quantities every rank
-  // agrees on.
+  // Tensor-core mode whenever the consumers' scans can run on the tensor cores: a launch plan exists for a whole
+  // sub-batch (n_ranks * sub_q queries; a ragged last sub-batch has fewer, and a plan that fits more queries fits
+  // fewer).  The choice uses only quantities every rank agrees on: whether a plan exists does not depend on the
+  // requested query tile (PIRB_TC_QT).  Otherwise the last-dimension entries travel as u64 limbs.
   const char* pk = getenv("PIRB_DIST_TC");
-  D.tc_mode = !(pk && pk[0] == '0') && c->tc.min_queries > 0 && tc_supported(c->P, last) &&
-              c->prm.num_pt / D.n_ranks >= c->tc.min_pt;
+  TcPlan plan;
+  D.tc_mode = !(pk && pk[0] == '0') && c->tc.min_queries > 0 && c->prm.num_pt / D.n_ranks >= c->tc.min_pt &&
+              tc_launch_plan(c->P, last, D.n_ranks * D.sub_q, &plan);
   const u64 slot_queries = (u64)D.n_sub * D.sub_q * D.n_ranks;
   const u64 head = ((u64)D.rows_per_rank + mid) * c->ctL;
   if (D.tc_mode) {

@@ -3,6 +3,7 @@
 #include <cuda_runtime.h>
 
 #include "pirb_common.h"
+#include "tc_plan.h"
 
 namespace pirb {
 
@@ -119,26 +120,28 @@ struct TcGeom {
   u32 kch;      // 128-byte K chunks
   u64 db_bytes; // size of the byte-planar database copy
 };
-bool tc_supported(const DevParams& P, u32 dimL);
+// launch plan (tc_plan.h) of a scan of n_queries queries over a last dimension of dimL entries, with the query tile
+// requested by PIRB_TC_QT; false when the device or the moduli rule the tensor cores out or no plan fits
+bool tc_launch_plan(const DevParams& P, u32 dimL, u32 n_queries, TcPlan* plan);
 void tc_geometry(const DevParams& P, u32 dimL, u32 n_rows, TcGeom* g);
-u64 tc_sv_bytes(const DevParams& P, const TcGeom& g, u32 n_queries, u32* qt_out, u32* n_qt_out);
+u64 tc_sv_bytes(const DevParams& P, const TcGeom& g, const TcPlan& plan);
 // u64 database [pt][k][N] -> byte-planar K-major copy dbT (db_bytes)
 cudaError_t launch_tc_pack_db(const DevParams& P, const u64* db, u64 num_pt, u32 dimL, u32 n_rows, const TcGeom& g,
                               u8* dbT, cudaStream_t st);
 // part[q][row][2][k][N] = sum_i1 sv[q][i1] (.) db[row*dimL + i1] mod q for a batch of queries (svT: scratch of
 // tc_sv_bytes; err_flag: device-visible int raised if the kernel's internal pipeline times out)
 // pack + scan for selection vectors held as u64 limbs [q][i1][2][k][N] (sv_qstride limbs between queries); svT: scratch
-// of tc_sv_bytes
-cudaError_t launch_tc_scan(const DevParams& P, const TcGeom& g, const u8* dbT, u32 dimL, u32 n_rows, const u64* sv,
-                           u64 sv_qstride, u32 n_queries, u8* svT, int* err_flag, int sm_count, u64* part,
+// of tc_sv_bytes; plan: tc_launch_plan for n_queries
+cudaError_t launch_tc_scan(const DevParams& P, const TcGeom& g, const TcPlan& plan, const u8* dbT, u32 dimL, u32 n_rows,
+                           const u64* sv, u64 sv_qstride, u32 n_queries, u8* svT, int* err_flag, int sm_count, u64* part,
                            cudaStream_t st);
 // the two halves: repack n_queries selection vectors into rows [row0, row0 + n_queries*2*nb) of an svT array with
 // rows_total rows per coefficient; scan against an svT array whose rows [row0, ...) hold the n_queries queries
 cudaError_t launch_tc_pack_sv(const DevParams& P, const TcGeom& g, const u64* sv, u64 sv_qstride, u32 dimL, u32 n_queries,
                               u8* svT, u32 rows_total, u32 row0, cudaStream_t st);
-cudaError_t launch_tc_scan_packed(const DevParams& P, const TcGeom& g, const u8* dbT, u32 dimL, u32 n_rows, const u8* svT,
-                                  u32 rows_total, u32 row0, u32 n_queries, int* err_flag, int sm_count, u64* part,
-                                  cudaStream_t st);
+cudaError_t launch_tc_scan_packed(const DevParams& P, const TcGeom& g, const TcPlan& plan, const u8* dbT, u32 n_rows,
+                                  const u8* svT, u32 rows_total, u32 row0, u32 n_queries, int* err_flag, int sm_count,
+                                  u64* part, cudaStream_t st);
 
 // ---- ciphertext-multiplication mode (kernels_ctmul.cu; database.cpp:202-211) ----
 // Evaluator::multiply [SEAL 3.5.6 bfv_multiply, BEHZ] split at its NTTs; n_batch independent problems, *_bstride apart.

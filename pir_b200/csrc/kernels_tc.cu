@@ -191,9 +191,7 @@ struct TcScanArgs {
   int* err;
 };
 
-constexpr int TC_MAX_ACC = 2;                            // accumulator buffers / epilogue groups (4 measured 7 % slower)
-constexpr int TC_THREADS = 128 + 128 * TC_MAX_ACC;       // 4 control warps + 4 warps per epilogue group
-constexpr u32 TC_A_STAGE_BYTES = 128 * 128;
+constexpr int TC_THREADS = 128 + 128 * TC_MAX_ACC;       // 4 control warps + 4 warps per epilogue group (tc_plan.h)
 
 template <int NB>
 __global__ void __launch_bounds__(TC_THREADS, 1)
@@ -439,11 +437,13 @@ void tc_geometry(const DevParams& P, u32 dimL, u32 n_rows, TcGeom* g) {
   g->db_bytes = (u64)P.k * P.N * g->ntiles * 128 * g->Kp;
 }
 
-bool tc_supported(const DevParams& P, u32 dimL) {
+bool tc_launch_plan(const DevParams& P, u32 dimL, u32 n_queries, TcPlan* plan) {
   TcGeom g;
   tc_geometry(P, dimL, 1, &g);
-  // s32 accumulators: dimL * 255^2 < 2^31; operand limbs: 5 or 6 bytes; the tile arithmetic below needs N % 32 == 0
-  return (g.nb == 5 || g.nb == 6) && dimL <= 32768 && encode_fn() != nullptr && (P.N % 64) == 0;
+  // the operand repacking works on 64-coefficient blocks; the tensor maps need the driver's encoder
+  if ((P.N % 64) != 0 || encode_fn() == nullptr) return false;
+  const char* want = std::getenv("PIRB_TC_QT");
+  return tc_plan(g.nb, dimL, n_queries, want ? atoi(want) : 16, plan);
 }
 
 cudaError_t launch_tc_pack_db(const DevParams& P, const u64* db, u64 num_pt, u32 dimL, u32 n_rows, const TcGeom& g,
@@ -456,16 +456,8 @@ cudaError_t launch_tc_pack_db(const DevParams& P, const u64* db, u64 num_pt, u32
   return cudaGetLastError();
 }
 
-u64 tc_sv_bytes(const DevParams& P, const TcGeom& g, u32 n_queries, u32* qt_out, u32* n_qt_out) {
-  // queries per MMA tile: a multiple of 8 (16 (q,p) pairs per epilogue piece), N = qt * 2 * nb <= 256
-  const u32 qpad = (n_queries + 7) / 8 * 8;
-  const u32 qt_max = g.nb == 5 ? 24 : 16;
-  int want = std::getenv("PIRB_TC_QT") ? atoi(std::getenv("PIRB_TC_QT")) : 16;
-  u32 qt = std::min<u32>(std::min<u32>(qpad, qt_max), (u32)std::max(8, want / 8 * 8));
-  const u32 n_qt = (qpad + qt - 1) / qt;
-  *qt_out = qt;
-  *n_qt_out = n_qt;
-  return (u64)P.k * P.N * n_qt * qt * 2 * g.nb * g.Kp;
+u64 tc_sv_bytes(const DevParams& P, const TcGeom& g, const TcPlan& plan) {
+  return (u64)P.k * P.N * plan.n_qt * plan.n_cols * g.Kp;
 }
 
 cudaError_t launch_tc_pack_sv(const DevParams& P, const TcGeom& g, const u64* sv, u64 sv_qstride, u32 dimL, u32 n_queries,
@@ -486,13 +478,11 @@ cudaError_t launch_tc_pack_sv(const DevParams& P, const TcGeom& g, const u64* sv
   return cudaGetLastError();
 }
 
-cudaError_t launch_tc_scan(const DevParams& P, const TcGeom& g, const u8* dbT, u32 dimL, u32 n_rows, const u64* sv,
-                           u64 sv_qstride, u32 n_queries, u8* svT, int* err_flag, int sm_count, u64* part,
+cudaError_t launch_tc_scan(const DevParams& P, const TcGeom& g, const TcPlan& plan, const u8* dbT, u32 dimL, u32 n_rows,
+                           const u64* sv, u64 sv_qstride, u32 n_queries, u8* svT, int* err_flag, int sm_count, u64* part,
                            cudaStream_t st) {
   const u32 kN = (u32)P.k * P.N;
-  u32 qt, n_qt;
-  tc_sv_bytes(P, g, n_queries, &qt, &n_qt);
-  const u32 sv_rows_total = n_qt * qt * 2 * g.nb;
+  const u32 sv_rows_total = plan.n_qt * plan.n_cols;
   // rows of padded queries must be zero; real ones are rewritten entirely (the K padding is never written)
   const u64 real_rows = (u64)n_queries * 2 * g.nb;
   if (real_rows < sv_rows_total) {
@@ -502,17 +492,16 @@ cudaError_t launch_tc_scan(const DevParams& P, const TcGeom& g, const u8* dbT, u
   }
   cudaError_t e = launch_tc_pack_sv(P, g, sv, sv_qstride, dimL, n_queries, svT, sv_rows_total, 0, st);
   if (e != cudaSuccess) return e;
-  return launch_tc_scan_packed(P, g, dbT, dimL, n_rows, svT, sv_rows_total, 0, n_queries, err_flag, sm_count, part, st);
+  return launch_tc_scan_packed(P, g, plan, dbT, n_rows, svT, sv_rows_total, 0, n_queries, err_flag, sm_count, part, st);
 }
 
-cudaError_t launch_tc_scan_packed(const DevParams& P, const TcGeom& g, const u8* dbT, u32 dimL, u32 n_rows, const u8* svT,
-                                  u32 sv_rows_total, u32 row0, u32 n_queries, int* err_flag, int sm_count, u64* part,
-                                  cudaStream_t st) {
-  (void)dimL;
+cudaError_t launch_tc_scan_packed(const DevParams& P, const TcGeom& g, const TcPlan& plan, const u8* dbT, u32 n_rows,
+                                  const u8* svT, u32 sv_rows_total, u32 row0, u32 n_queries, int* err_flag, int sm_count,
+                                  u64* part, cudaStream_t st) {
   const u32 kN = (u32)P.k * P.N;
-  u32 qt, n_qt;
-  tc_sv_bytes(P, g, n_queries, &qt, &n_qt);
-  const u32 n_cols = qt * 2 * g.nb;
+  const u32 n_cols = plan.n_cols;
+  if (plan.Kp != g.Kp || plan.kch != g.kch || n_cols != plan.qt * 2 * g.nb || plan.n_qt * plan.qt < n_queries)
+    return cudaErrorInvalidValue;  // a plan made for another shape
 
   CUtensorMap mapA, mapB;
   if (!make_map(&mapA, dbT, (u64)kN * g.ntiles * 128, g.Kp, 128)) return cudaErrorInvalidValue;
@@ -526,22 +515,17 @@ cudaError_t launch_tc_scan_packed(const DevParams& P, const TcGeom& g, const u8*
   A.Kp = g.Kp;
   A.kch = g.kch;
   A.n_queries = n_queries;
-  A.n_qt = n_qt;
-  A.qt = qt;
+  A.n_qt = plan.n_qt;
+  A.qt = plan.qt;
   A.n_cols = n_cols;
   A.sv_rows_total = sv_rows_total;
   A.sv_row0 = row0;
   A.part = part;
   A.err = err_flag;
-  const size_t b_buf = (size_t)g.kch * n_cols * 128;
-  const size_t e_bytes = (size_t)TC_MAX_ACC * 16 * 128 * 8 * (g.nb <= 5 ? 1 : 2);
   A.n_acc = (TC_MAX_ACC >= 4 && 4 * n_cols <= 512) ? 4 : 2;  // accumulator buffers must fit the 512 TMEM columns
-  const size_t fixed = e_bytes + 1024;  // barriers, TMEM slot, alignment slack
-  const size_t budget = 227 * 1024;
-  A.b_bufs = (2 * b_buf + fixed + 4 * TC_A_STAGE_BYTES <= budget) ? 2 : 1;
-  if (A.b_bufs * b_buf + fixed + 2 * TC_A_STAGE_BYTES > budget) return cudaErrorInvalidConfiguration;
-  A.stages = (u32)std::min<size_t>(8, (budget - fixed - A.b_bufs * b_buf) / TC_A_STAGE_BYTES);
-  const size_t smem = (size_t)A.stages * TC_A_STAGE_BYTES + A.b_bufs * b_buf + fixed;
+  A.b_bufs = plan.b_bufs;
+  A.stages = plan.stages;
+  const size_t smem = plan.smem;
   const int grid = std::min<int>(sm_count, (int)kN);
   auto go = [&](auto kern) -> cudaError_t {
     cudaError_t e2 = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);

@@ -42,6 +42,7 @@ static inline size_t __cvta_generic_to_shared(const void* p) { return (size_t)p;
 #include "../../oracle/pir_oracle.hpp"
 #include "../../pir_b200/csrc/host_math.h"
 #include "../../pir_b200/csrc/pirb_device.cuh"
+#include "../../pir_b200/csrc/tc_plan.h"
 
 typedef unsigned __int128 u128;
 typedef __int128 i128;
@@ -270,8 +271,85 @@ static int check_galois(std::mt19937_64& rng) {
   return 0;
 }
 
+// The launch plan of the tensor-core batched scan (tc_plan.h) for every shape it can be asked for: each plan it accepts
+// must be launchable and exact, it must take the widest query tile that fits, and it may refuse only when not even the
+// narrowest tile fits.  The plans of the benchmark workloads are pinned: those scans launch exactly as they did before
+// the plan was factored out.
+static int check_tc_plans() {
+  const uint32_t A = pirb::TC_A_STAGE_BYTES, budget = pirb::TC_SMEM_BUDGET;
+  long accepted = 0;
+  for (uint32_t nb : {5u, 6u}) {
+    const uint32_t fixed = pirb::TC_MAX_ACC * 16 * 128 * 8 * (nb == 5 ? 1 : 2) + 1024;
+    const uint32_t dimL_max = nb == 5 ? 2048 : 1280;  // kch 16 / 10: the last B operand of qt 8 that fits
+    for (int req : {8, 16, 24}) {
+      for (uint32_t dimL = 1; dimL <= 33000; ++dimL) {
+        pirb::TcPlan prev = {};
+        bool prev_ok = true;
+        for (uint32_t nq = 1; nq <= 64; ++nq) {
+          pirb::TcPlan p;
+          const bool ok = pirb::tc_plan(nb, dimL, nq, req, &p);
+          CHECK(ok == (dimL <= dimL_max), "plan existence (nb %u, dimL %u, %u queries, qt %d): %d", nb, dimL, nq, req, ok);
+          if (!ok) continue;
+          ++accepted;
+          CHECK(prev_ok, "a plan for %u queries but none for fewer (nb %u, dimL %u)", nq, nb, dimL);
+          CHECK(p.smem <= budget && p.stages >= 2 && p.stages <= 8, "shared memory %u B, %u stages (nb %u, dimL %u, %u q)",
+                p.smem, p.stages, nb, dimL, nq);
+          CHECK(p.qt % 8 == 0 && p.qt >= 8 && (int)p.qt <= std::max(8, req / 8 * 8), "qt %u for requested %d", p.qt, req);
+          CHECK(p.n_cols == p.qt * 2 * nb && p.n_cols % 16 == 0 && p.n_cols <= 256, "MMA N %u (nb %u, qt %u)", p.n_cols, nb,
+                p.qt);
+          CHECK(p.n_qt * p.qt >= nq && (p.n_qt - 1) * p.qt < nq, "%u tiles of %u queries for %u queries", p.n_qt, p.qt, nq);
+          CHECK(p.Kp >= dimL && p.Kp % 16 == 0 && p.Kp < dimL + 16 && p.kch * 128 >= p.Kp && (p.kch - 1) * 128 < p.Kp,
+                "K geometry Kp %u kch %u for dimL %u", p.Kp, p.kch, dimL);
+          CHECK((uint64_t)dimL * 255 * 255 < (1ull << 31), "s32 accumulator bound at dimL %u", dimL);
+          const uint32_t b_buf = p.kch * p.n_cols * 128;
+          CHECK(p.smem == p.stages * A + p.b_bufs * b_buf + fixed, "shared memory accounting");
+          CHECK(p.b_bufs == ((2 * b_buf + fixed + 4 * A <= budget) ? 2u : 1u), "b_bufs %u (nb %u, dimL %u, qt %u)", p.b_bufs,
+                nb, dimL, p.qt);
+          CHECK(p.stages == std::min<uint32_t>(8, (budget - fixed - p.b_bufs * b_buf) / A), "A ring depth");
+          // widest tile: the next wider one allowed by the request and the query count would not fit
+          const uint32_t cap = std::min(std::min((nq + 7) / 8 * 8, nb == 5 ? 24u : 16u), (uint32_t)std::max(8, req / 8 * 8));
+          if (p.qt < cap)
+            CHECK(p.kch * (p.qt + 8) * 2 * nb * 128 + fixed + 2 * A > budget, "qt %u chosen although %u fits (dimL %u)",
+                  p.qt, p.qt + 8, dimL);
+          else
+            CHECK(p.qt == cap, "qt %u above the cap %u", p.qt, cap);
+          if (nq > 1) CHECK(p.qt >= prev.qt, "qt shrinks from %u to %u as queries grow", prev.qt, p.qt);
+          prev = p;
+          prev_ok = ok;
+        }
+      }
+    }
+  }
+  // the shapes that used to be refused at launch: a narrower tile now
+  pirb::TcPlan p;
+  CHECK(pirb::tc_plan(5, 1024, 16, 16, &p) && p.qt == 16, "nb 5 dimL 1024");
+  CHECK(pirb::tc_plan(5, 1025, 9, 16, &p) && p.qt == 8 && p.n_qt == 2, "nb 5 dimL 1025");
+  CHECK(pirb::tc_plan(5, 640, 24, 24, &p) && p.qt == 24, "nb 5 dimL 640 qt 24");
+  CHECK(pirb::tc_plan(5, 641, 24, 24, &p) && p.qt == 16 && p.n_qt == 2, "nb 5 dimL 641 qt 24");
+  CHECK(pirb::tc_plan(6, 640, 16, 16, &p) && p.qt == 16, "nb 6 dimL 640");
+  CHECK(pirb::tc_plan(6, 641, 9, 16, &p) && p.qt == 8 && p.n_qt == 2, "nb 6 dimL 641");
+  CHECK(!pirb::tc_plan(6, 1281, 4, 16, &p) && !pirb::tc_plan(5, 2049, 4, 16, &p), "beyond the narrowest tile");
+  // benchmark workloads (default PIRB_TC_QT): configs[3] (N=4096, dims [333, 332]) with 8 queries on one GPU and 16 / 64
+  // per scan on several; configs[4] d=2 (N=4096, [665, 664]) with 8 and 16; configs[2] (N=8192, [235, 235]) with 4..16
+  struct Want { uint32_t nb, dimL, nq, qt, n_qt, kch, b_bufs, stages, smem; };
+  const Want bench[] = {{5, 332, 8, 8, 1, 3, 2, 8, 226304},  {5, 332, 16, 16, 1, 3, 2, 4, 222208},
+                        {5, 332, 64, 16, 4, 3, 2, 4, 222208}, {5, 664, 8, 8, 1, 6, 2, 4, 222208},
+                        {5, 664, 16, 16, 1, 6, 1, 4, 222208}, {6, 235, 4, 8, 1, 2, 2, 7, 230400},
+                        {6, 235, 8, 8, 1, 2, 2, 7, 230400},   {6, 235, 16, 16, 1, 2, 2, 4, 230400}};
+  for (const Want& w : bench) {
+    CHECK(pirb::tc_plan(w.nb, w.dimL, w.nq, 16, &p), "bench plan missing (dimL %u, %u queries)", w.dimL, w.nq);
+    CHECK(p.qt == w.qt && p.n_qt == w.n_qt && p.kch == w.kch && p.b_bufs == w.b_bufs && p.stages == w.stages &&
+              p.smem == w.smem,
+          "bench plan changed (dimL %u, %u queries): qt %u n_qt %u kch %u b_bufs %u stages %u smem %u", w.dimL, w.nq, p.qt,
+          p.n_qt, p.kch, p.b_bufs, p.stages, p.smem);
+  }
+  std::printf("tensor-core scan plans: %ld accepted shapes launchable and exact, benchmark plans unchanged\n", accepted);
+  return 0;
+}
+
 int main() {
   std::mt19937_64 rng(2024);
+  if (check_tc_plans()) return 1;
   // BFVDefault primes of N=4096 / N=8192, the 24-bit-plain config's moduli are the same; plus a 44-bit prime (the
   // largest the FP64 engine accepts)
   std::vector<u64> moduli;

@@ -2,6 +2,7 @@
 oracle on the same seeded inputs — bit-exact on all limbs — plus decrypt-level checks against the reference's
 known-answer vectors and size-independent properties at BASELINE.json's sizes.
 """
+import dataclasses
 import json
 import os
 
@@ -694,10 +695,19 @@ def test_device_populate_and_shard_file_roundtrip(tmp_path):
 
 
 # ------------------------------------------------------------------------------------------------ NVLink exchange flow
-@pytest.mark.parametrize("dbsize,world,ql,sub,packed", [(82, 2, 2, 1, 0), (82, 3, 3, 2, 0), (300, 4, 4, 0, 0), (3, 4, 1, 0, 0),
-                                                        (300, 2, 5, 2, 0), (300, 2, 5, 2, 1), (82, 3, 3, 2, 1),
-                                                        (300, 4, 2, 0, 1)])
-def test_peer_memory_exchange_flow_matches_oracle(dbsize, world, ql, sub, packed, monkeypatch):
+_PEER_FLOW = [(82, 2, 2, 1, 0), (82, 3, 3, 2, 0), (300, 4, 4, 0, 0), (3, 4, 1, 0, 0), (300, 2, 5, 2, 0), (300, 2, 5, 2, 1),
+              (82, 3, 3, 2, 1), (300, 4, 2, 0, 1)]
+# tensor-core exchange geometries: 20 queries per scan (two query tiles); a last dimension of 400 (four K chunks, one
+# B buffer); empty shards; a last dimension of 1100, whose B operand fits only with 8-query tiles
+_PEER_FLOW_TC = [(300, 4, 5, 5, 1, None), (1350, 2, 5, 5, 1, [4, 400]), (3, 4, 1, 0, 1, None),
+                 (2150, 2, 5, 5, 1, [2, 1100])]
+
+
+@pytest.mark.parametrize("dbsize,world,ql,sub,packed,dims",
+                         [pytest.param(*r, None, id="-".join(map(str, r))) for r in _PEER_FLOW] +
+                         [pytest.param(*r, id="-".join(map(str, r[:5])) + ("" if r[5] is None else "-dims%dx%d" % tuple(r[5])))
+                          for r in _PEER_FLOW_TC])
+def test_peer_memory_exchange_flow_matches_oracle(dbsize, world, ql, sub, packed, dims, monkeypatch):
     """pirb_dist_*: the row-sharded flow whose exchange is done by the kernels over peer memory (selection-vector NTT
     storing into every rank's slot, per-sub-batch flags, partial replies added by peer loads).  All ranks live in this
     process and on this one GPU (ShardGroup), which exercises exactly the kernels, flags and slot arithmetic of the
@@ -718,6 +728,8 @@ def test_peer_memory_exchange_flow_matches_oracle(dbsize, world, ql, sub, packed
     n = 4096
     ep = pb.GenerateEncryptionParams(n, 20)
     p = pb.CreatePIRParameters(dbsize, 0, 2, ep)
+    if dims is not None:  # explicit dimensions: a long last dimension over a small database
+        p = dataclasses.replace(p, dimensions=list(dims))
     mods = list(ep.coeff_modulus)
     k = len(mods) - 1
     rng = np.random.default_rng(dbsize * 31 + world)
@@ -880,10 +892,14 @@ def test_ct_multiply_mode_db_multiply_matches_oracle(n, bits, dbsize, d, idx):
 @pytest.mark.parametrize("n,bits,elem,bpc,dbsize,d,indices",
                          [(4096, 24, 0, 0, 10, 1, [0]), (4096, 16, 0, 10, 9, 2, [1, 5]),
                           (4096, 16, 0, 6, 500, 2, [9, 125]), (8192, 42, 0, 0, 87, 2, [5, 33, 86]),
-                          (4096, 16, 64, 10, 1200, 1, [0, 80, 81, 123, 777, 1199])])
-def test_ct_multiply_mode_end_to_end_matches_oracle(n, bits, elem, bpc, dbsize, d, indices):
+                          (4096, 16, 64, 10, 1200, 1, [0, 80, 81, 123, 777, 1199]),
+                          (4096, 16, 0, 6, 500, 2, [9, 125, 0, 250, 499])])
+def test_ct_multiply_mode_end_to_end_matches_oracle(n, bits, elem, bpc, dbsize, d, indices, monkeypatch):
     """correctness_test.cpp:94-105 (use_ciphertext_multiplication == true): client -> PIRServer::ProcessRequest ->
-    client, every reply bit-exact against the oracle, the whole batch of queries in one device call."""
+    client, every reply bit-exact against the oracle, the whole batch of queries in one device call.  A batch of 4 or
+    more queries at d >= 2 takes the tensor-core last-dimension scan, here even on a small database."""
+    if d >= 2 and len(indices) >= 4:
+        monkeypatch.setenv("PIRB_TC_MIN_PT", "0")
     p = _params(dbsize, elem, d, n, bits, bpc, ct_mult=True)
     cl = _harness(p, seed=5)
     items = _random_items(p)
