@@ -13,6 +13,7 @@
 // polynomials never touch global memory and a tree level costs one launch instead of three.
 #include <cooperative_groups.h>
 
+#include <algorithm>
 #include <cstdlib>
 
 #include <type_traits>
@@ -134,8 +135,12 @@ k_ks_level_cluster(const __grid_constant__ DevParams P, u64* __restrict__ work, 
     }
   }
   if constexpr (TWS) {
-    // every forward pass has ended with a block barrier: the table buffer is free for the inverse twiddles
+    // every forward pass has ended with a block barrier: the table buffer is free for the inverse twiddles.  A CTA
+    // without digits (c = 1 when k = 1) has not waited for the forward table yet; its copy must have landed before
+    // the barrier is armed again and the buffer rewritten (otherwise two copies race into it and the second arrival
+    // lands on a phase that is still pending).
     if (tid == 0) {
+      mbar_wait(twbar, 0);
       asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
       mbar_expect_tx(twbar, N * 8);
       bulk_g2s_plain(TWb, mI.iw1, N * 8, twbar);
@@ -524,15 +529,23 @@ k_ks_level_cluster2(const __grid_constant__ DevParams P, u64* __restrict__ work,
   }
 }
 
-static size_t ks_cluster_smem(const DevParams& P) {
-  const bool tws = P.ntt_engine == ENG_FP64 && P.logn <= 12;  // + staged twiddle table and its mbarrier
-  return (size_t)((P.k + 1) / 2 + 1 + (tws ? 1 : 0)) * P.N * sizeof(u64) + (tws ? 16 : 0);
+static size_t ks_cluster_smem(int k, int logn, int engine) {
+  const bool tws = engine == ENG_FP64 && logn <= 12;  // + staged twiddle table and its mbarrier
+  return (size_t)((k + 1) / 2 + 1 + (tws ? 1 : 0)) * ((size_t)1 << logn) * sizeof(u64) + (tws ? 16 : 0);
 }
 
-bool ks_cluster_supported(const DevParams& P) {
-  const int k = P.k;
-  const size_t smem = ks_cluster_smem(P);
-  return 2 * (k + 1) <= 16 && smem <= 227 * 1024 && P.logn >= 11 && P.logn <= 14;
+static bool ks_cluster_fits(int k, int logn, int engine) {
+  return 2 * (k + 1) <= 16 && ks_cluster_smem(k, logn, engine) <= 227 * 1024 && logn >= 11 && logn <= 14;
+}
+
+bool ks_cluster_supported(const DevParams& P) { return ks_cluster_fits(P.k, P.logn, P.ntt_engine); }
+
+// the most dynamic shared memory any supported k needs at this N and engine (k selects no instantiation of its own)
+static size_t ks_cluster_smem_max(int logn, int engine) {
+  size_t most = 0;
+  for (int k = 1; 2 * (k + 1) <= 16; ++k)
+    if (ks_cluster_fits(k, logn, engine)) most = std::max(most, ks_cluster_smem(k, logn, engine));
+  return most;
 }
 
 // second generation: FP64 engine, staged twiddles (N <= 4096), k <= 2 (k digit buffers + table fit twice per SM)
@@ -592,23 +605,25 @@ cudaError_t launch_ks_level_cluster(const DevParams& P, u64* work, const LevelAr
     }
   }
   const unsigned csize = 2 * (k + 1);
-  const size_t smem = ks_cluster_smem(P);
+  const size_t smem = ks_cluster_smem(k, P.logn, P.ntt_engine);
   auto go = [&](auto ln, auto lz, auto mm) -> cudaError_t {
     constexpr int LN = decltype(ln)::value;
     constexpr int LZ = decltype(lz)::value;
     constexpr int MM = decltype(mm)::value;
     auto kern = k_ks_level_cluster<LN, LZ, MM>;
-    static size_t configured[64] = {};  // per device: largest dynamic shared memory size already set
+    // Every k shares this instantiation, so it is configured once per device for the largest of them: the most shared
+    // memory any k needs and clusters above the portable 8 CTAs (k >= 4).  A process may serve several parameter sets
+    // in any order; k = 3 and k = 4 need the same bytes, and only the larger cluster needs the opt-in.
+    static bool configured[64] = {};
     int dev = 0;
     cudaGetDevice(&dev);
-    if (configured[dev & 63] < smem) {
-      cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (!configured[dev & 63]) {
+      cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                           (int)ks_cluster_smem_max(LN, LZ));
       if (e != cudaSuccess) return e;
-      if (csize > 8) {
-        e = cudaFuncSetAttribute(kern, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
-        if (e != cudaSuccess) return e;
-      }
-      configured[dev & 63] = smem;
+      e = cudaFuncSetAttribute(kern, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
+      if (e != cudaSuccess) return e;
+      configured[dev & 63] = true;
     }
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(nodes * csize);

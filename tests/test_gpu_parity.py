@@ -587,7 +587,7 @@ def _find_ntt_primes(bits, n, count):
 
 
 @pytest.mark.parametrize("n,bits,label", [(4096, 60, "60-bit moduli: corrected integer butterflies + 128-bit MACs"),
-                                           (4096, 50, "50-bit moduli: lazy integer butterflies + 128-bit MACs"),
+                                           (4096, 50, "50-bit moduli: corrected integer butterflies + 128-bit MACs"),
                                            (4096, 47, "47-bit moduli: lazy integer butterflies + 24-bit-split MACs"),
                                            (2048, 40, "N=2048 with two data moduli: FP64 engine at another size"),
                                            (16384, 44, "N=16384, k=3: FP64 engine, 128 KiB transforms")])
