@@ -10,7 +10,7 @@ HDRS := $(wildcard $(SRC)/*.h $(SRC)/*.cuh) include/pir_b200.h
 
 WIRE := pir_b200/lib/libpirb_wire.so
 
-all: $(LIB) $(WIRE) oracle build/shim_test build/shim_host_test build/wire_test build/wire_fuzz_test build/device_math_host_test build/ctmul_host_test build/shim_bench
+all: $(LIB) $(WIRE) oracle build/shim_test build/shim_host_test build/wire_test build/wire_fuzz_test build/device_math_host_test build/ctmul_host_test build/shim_bench build/multi_client_test
 
 $(OBJ)/%.o: $(SRC)/%.cu $(HDRS)
 	@mkdir -p $(OBJ)
@@ -30,6 +30,11 @@ $(WIRE): pir_b200/cpp/wire_capi.cpp pir_b200/cpp/wire.hpp
 build/shim_test: tests/cpp/shim_test.cpp pir_b200/cpp/pir_b200.hpp pir_b200/cpp/wire.hpp oracle/pir_oracle.hpp oracle/bfv_mul_oracle.hpp include/pir_b200.h $(LIB)
 	@mkdir -p build
 	g++ -O2 -std=c++17 -march=x86-64-v3 -o $@ tests/cpp/shim_test.cpp -Lpir_b200/lib -lpirb200 -Wl,-rpath,'$$ORIGIN/../pir_b200/lib'
+
+# C++ ProcessRequests (queries of several clients in one batched pass) against per-request ProcessRequest and the oracle
+build/multi_client_test: tests/cpp/multi_client_test.cpp pir_b200/cpp/pir_b200.hpp pir_b200/cpp/wire.hpp oracle/pir_oracle.hpp include/pir_b200.h $(LIB)
+	@mkdir -p build
+	g++ -O2 -std=c++17 -march=x86-64-v3 -Wall -o $@ tests/cpp/multi_client_test.cpp -Lpir_b200/lib -lpirb200 -Wl,-rpath,'$$ORIGIN/../pir_b200/lib'
 
 # the reference-facing C++ call timed like pir/cpp/benchmark.cpp (bench.py runs it and reports e2e_cpp / e2e_wire)
 build/shim_bench: tools/shim_bench.cpp pir_b200/cpp/pir_b200.hpp pir_b200/cpp/wire.hpp include/pir_b200.h $(LIB)

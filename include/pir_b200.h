@@ -114,6 +114,14 @@ int pirb_db_multiply(pirb_ctx* ctx, uint64_t* sv, uint64_t n_sv, uint64_t* out, 
  * (cudaHostAlloc / cudaHostRegister) are read and written in place by the kernels, pageable ones are staged. */
 int pirb_answer(pirb_ctx* ctx, const pirb_keys* keys, const uint64_t* queries, uint32_t n_queries, uint64_t n_ct,
                 uint64_t* replies);
+/* PIRServer::processQuery for queries of several clients in one pass: keys[i] is the Galois-key handle of query i
+ * (handles may repeat, in any order).  Same buffers, layouts, status codes and zero-copy rules as pirb_answer /
+ * pirb_answer_dev.  Unsharded, re-encoder contexts only (3 otherwise).  Every handle is checked before anything runs:
+ * 3 for a null handle or one loaded on a context of another shape, 13 for a handle that lacks the Galois element of
+ * an expansion level; the message names the query, and no reply is written.  pirb_answer_multi_dev returns before the
+ * device has read the handles' keys: the caller must not destroy a handle while such a call that uses it is in flight. */
+int pirb_answer_multi(pirb_ctx* ctx, const pirb_keys* const* keys, const uint64_t* queries, uint32_t n_queries,
+                      uint64_t n_ct, uint64_t* replies);
 
 /* ---- Ciphertext-multiplication mode (PIRParameters.use_ciphertext_multiplication; contexts created with the flag).
  * The upper dimensions multiply the lower result with the selection ciphertext by Evaluator::multiply and, when the
@@ -144,6 +152,9 @@ int pirb_answer_dev(pirb_ctx* ctx, const pirb_keys* keys, const uint64_t* d_quer
                     uint64_t n_ct, uint64_t* d_replies, void* stream);
 int pirb_answer_partial_dev(pirb_ctx* ctx, const pirb_keys* keys, const uint64_t* d_queries, uint32_t n_queries,
                             uint64_t n_ct, uint64_t* d_partial, void* stream);
+/* pirb_answer_dev with one Galois-key handle per query (see pirb_answer_multi) */
+int pirb_answer_multi_dev(pirb_ctx* ctx, const pirb_keys* const* keys, const uint64_t* d_queries, uint32_t n_queries,
+                          uint64_t n_ct, uint64_t* d_replies, void* stream);
 /* The two halves of pirb_answer_partial_dev, for batches whose expansion is split by query across ranks:
  * pirb_expand_ntt_dev: oblivious expansion (server.cpp:148-171) + the selection-vector NTT (database.cpp:190,222)
  *   -> d_sv_ntt[n_queries][dim_sum][2][k][N];

@@ -63,6 +63,9 @@ SYMBOLS = {
     "pirb_expand": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_int, C.c_void_p]),
     "pirb_db_multiply": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64, u64p]),
     "pirb_answer": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint64, C.c_void_p]),
+    "pirb_answer_multi": (C.c_int, [C.c_void_p, C.POINTER(C.c_void_p), C.c_void_p, C.c_uint32, C.c_uint64, C.c_void_p]),
+    "pirb_answer_multi_dev": (C.c_int, [C.c_void_p, C.POINTER(C.c_void_p), C.c_void_p, C.c_uint32, C.c_uint64, C.c_void_p,
+                                        C.c_void_p]),
     "pirb_relin_keys_load": (C.c_int, [C.c_void_p, C.c_void_p, C.POINTER(C.c_void_p)]),
     "pirb_reply_polys": (C.c_uint32, [C.c_void_p, C.c_int]),
     "pirb_db_multiply_ct": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p, C.c_uint64, u32p]),

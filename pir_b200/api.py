@@ -10,6 +10,7 @@ pir/cpp/parameters.h:40-75, with SEAL objects replaced by raw RNS limbs (numpy u
 absl::Status codes surface as PIRStatusError(code): 3 = InvalidArgument, 13 = Internal.
 """
 import ctypes as C
+from collections import OrderedDict
 from dataclasses import dataclass, field
 from typing import List, Optional, Sequence
 
@@ -481,6 +482,9 @@ class PIRServer:
         self.ctx = db.ctx  # device state is shared with the database it serves
         self._key_cache = (None, None)
         self._relin_cache = (None, None)
+        # ProcessRequests: key handles of recent clients, least recently used first, keyed on the GaloisKeys object
+        self.key_cache_capacity = 16
+        self._multi_key_cache = OrderedDict()  # id(GaloisKeys) -> (GaloisKeys, _KeyHandle)
 
     @classmethod
     def Create(cls, db: PIRDatabase, params: PIRParameters):
@@ -543,6 +547,68 @@ class PIRServer:
         out = out.reshape(shape)
         resp.reply = [out[i] for i in range(n_q)]
         return resp
+
+    def _trim_key_cache(self, keep=()):
+        """Close the least recently used handles beyond key_cache_capacity, except those in `keep`: closing a handle
+        frees its keys on the device, so the handles of a batch stay open until its call has returned."""
+        over = len(self._multi_key_cache) - max(1, int(self.key_cache_capacity))
+        for key in list(self._multi_key_cache):
+            if over <= 0:
+                break
+            if key not in keep:
+                self._multi_key_cache.pop(key)[1].close()
+                over -= 1
+
+    def _batch_keys(self, gks):
+        """One handle per GaloisKeys object of the batch (cached across calls), in batch order."""
+        handles, used = [], set()
+        for gk in gks:
+            key = id(gk)  # the cache holds the object, so its id is not reused while the entry lives
+            if key in self._multi_key_cache:
+                self._multi_key_cache.move_to_end(key)
+            else:
+                self._multi_key_cache[key] = (gk, _KeyHandle(self.ctx, gk))
+            used.add(key)
+            self._trim_key_cache(keep=used)
+            handles.append(self._multi_key_cache[key][1])
+        return handles
+
+    def ProcessRequests(self, requests: List[Request]) -> List[Response]:
+        """ProcessRequest for requests of several clients, each with its own Galois keys, in one batched device call
+        (pirb_answer_multi): the Response of each request equals what ProcessRequest returns for it alone.  Key handles
+        come from an LRU of key_cache_capacity clients keyed on the GaloisKeys object.  In ciphertext-multiplication
+        mode the requests are answered one by one."""
+        requests = list(requests)
+        for r in requests:
+            if r.galois_keys is None:
+                raise PIRStatusError(INVALID_ARGUMENT, "galois keys missing")
+        if getattr(self.ctx, "ct_mode", False):
+            return [self.ProcessRequest(r) for r in requests]
+        n_ct = self.ctx.query_cts
+        for r in requests:
+            if any(q.size // self.ctx.ct_limbs != n_ct for q in r.query):
+                raise PIRStatusError(INVALID_ARGUMENT,
+                                     "Number of ciphertexts doesn't match number of items for oblivious expansion.")
+        shape = (n_ct, 2, self.ctx.k, self.ctx.N)
+        queries = [np.asarray(q).reshape(shape) for r in requests for q in r.query]
+        owners = [r.galois_keys for r in requests for _ in r.query]
+        n_q = len(queries)
+        if not n_q:
+            return [Response() for _ in requests]
+        q = _u64(np.stack(queries))
+        out = np.empty((n_q, self.ctx.reply_cts, 2, self.ctx.k, self.ctx.N), dtype=np.uint64)
+        try:
+            handles = self._batch_keys(owners)
+            table = (C.c_void_p * n_q)(*[h.h.value for h in handles])
+            _check(_lib.lib().pirb_answer_multi(self.ctx.h, table, C.c_void_p(q.ctypes.data), n_q, n_ct,
+                                                C.c_void_p(out.ctypes.data)))
+        finally:
+            self._trim_key_cache()
+        res, i = [], 0
+        for r in requests:
+            res.append(Response(reply=[out[i + j] for j in range(len(r.query))]))
+            i += len(r.query)
+        return res
 
     def ProcessRequestBytes(self, serialized_request: bytes) -> bytes:
         """server.cpp:44-65 on the wire: a serialized pir.Request (protobuf framing, SEAL 3.5.6 objects, seed-compressed

@@ -12,6 +12,7 @@
 #include <cstring>
 #include <map>
 #include <memory>
+#include <optional>
 #include <string>
 #include <tuple>
 #include <vector>
@@ -139,6 +140,9 @@ struct pirb_ctx {
   bool ev_last_valid = false;
   std::vector<DevBuf> tables;
   DevBuf db, stage, work, dig, acc, xch, part, bufA[2], pts, qbuf, rbuf, svbuf;
+  // key pointers of the calls with per-query Galois keys (pirb_answer_multi*): [tree level][query], uploaded before the
+  // call's first launch; captured graphs read it at its fixed address, so one graph serves every mix of clients
+  DevBuf ktab;
   std::map<std::tuple<u64, int, int, int>, std::unique_ptr<ExpandPlan>> plans;  // (items, single, first tree, trees)
   bool profiling = false;
   cudaEvent_t ev[PIRB_N_STAGES + 1] = {};
@@ -212,7 +216,7 @@ struct pirb_ctx {
     u64 work_bytes = 4ull << 30;  // products of a level are formed for as many queries at a time as fit this budget
   } ct;
   pirb_ctx() {
-    for (DevBuf* b : {&db, &stage, &work, &dig, &acc, &xch, &part, &bufA[0], &bufA[1], &pts, &qbuf, &rbuf, &svbuf, &dbg,
+    for (DevBuf* b : {&db, &stage, &work, &dig, &acc, &xch, &part, &bufA[0], &bufA[1], &pts, &qbuf, &rbuf, &svbuf, &ktab, &dbg,
                       &dist.peer_table, &dist.self_table, &dist.stage, &tc.dbT, &tc.svT})
       b->epoch = &alloc_epoch;
   }
@@ -300,8 +304,11 @@ ExpandPlan* get_plan(pirb_ctx* c, u64 total_items, int single, int* rc, int t_fi
 // lvl_lo / lvl_hi and q_first / q_count restrict the call to tree levels [lvl_lo, lvl_hi) of queries
 // [q_first, q_first + q_count) of the batch (the workspaces are always sized for the whole batch): the multi-GPU flow
 // runs the small top levels for all queries at once and the wide bottom levels per sub-batch.
+// key_table: every query has its own Galois keys, whose pointers c->ktab holds ([level][n_queries], see
+// multi_key_table); `keys` is unused.
 int run_expand(pirb_ctx* c, const pirb_keys* keys, ExpandPlan* pl, const u64* d_query, int n_queries,
-               cudaStream_t st, int lvl_lo = 0, int lvl_hi = -1, int q_first = 0, int q_count = -1) {
+               cudaStream_t st, int lvl_lo = 0, int lvl_hi = -1, int q_first = 0, int q_count = -1,
+               bool key_table = false) {
   const u64 q_stride = 2 * pl->cap * c->ctL;
   if (lvl_hi < 0) lvl_hi = pl->max_logm;
   if (q_count < 0) q_count = n_queries - q_first;
@@ -319,9 +326,12 @@ int run_expand(pirb_ctx* c, const pirb_keys* keys, ExpandPlan* pl, const u64* d_
                                  (u64)pl->n_ct_in * c->ctL, work, pl->d_off.p, pl->n_trees, q_count, q_stride, st));
   for (int j = lvl_lo; j < lvl_hi; ++j) {
     const u32 g = (c->N >> j) + 1;
-    if (!keys) return fail(PIRB_INTERNAL, "Galois keys required");
-    const u64* key = keys->find(g);
-    if (!key) return fail(PIRB_INTERNAL, "Galois key not present for element " + std::to_string(g));
+    const u64* key = nullptr;
+    if (!key_table) {
+      if (!keys) return fail(PIRB_INTERNAL, "Galois keys required");
+      key = keys->find(g);
+      if (!key) return fail(PIRB_INTERNAL, "Galois key not present for element " + std::to_string(g));
+    }
     LevelArgs L;
     L.src_off = pl->d_off.p + pl->lvl_src[j];
     L.dst_off = pl->d_off.p + pl->lvl_dst[j];
@@ -331,6 +341,7 @@ int run_expand(pirb_ctx* c, const pirb_keys* keys, ExpandPlan* pl, const u64* d_
     L.g = g;
     L.q_stride = q_stride;
     L.n_queries = q_count;
+    L.key_tab = key_table ? reinterpret_cast<const u64* const*>(c->ktab.p) + (size_t)j * n_queries + q_first : nullptr;
     L.xch = c->xch.p;
     L.dbg = !c->dbg.p ? nullptr : (c->dbg_level == -2 ? c->dbg.p + (size_t)j * 65536 : (j == c->dbg_level ? c->dbg.p : nullptr));
     L.dbg_clock = (c->dbg_level >= 0 && getenv("PIRB_STAMP_CLOCK")) ? atoi(getenv("PIRB_STAMP_CLOCK")) : 0;
@@ -339,7 +350,7 @@ int run_expand(pirb_ctx* c, const pirb_keys* keys, ExpandPlan* pl, const u64* d_
       LAUNCH(c, launch_ks_level_cluster(c->P, work, L, key, 0, st));
     } else {
       LAUNCH(c, launch_ks_digits(c->P, work, L, c->dig.p, st));
-      LAUNCH(c, launch_ks_mac_intt(c->P, c->dig.p, key, c->acc.p, n_nodes, st));
+      LAUNCH(c, launch_ks_mac_intt(c->P, c->dig.p, key, c->acc.p, n_nodes, st, L.key_tab, (u32)L.n_trees << j));
       LAUNCH(c, launch_ks_combine(c->P, work, L, c->acc.p, 0, st));
     }
   }
@@ -667,7 +678,7 @@ int run_multiply_ct(pirb_ctx* c, const pirb_keys* relin, const u64* d_sv, u64 sv
 }
 
 int run_answer(pirb_ctx* c, const pirb_keys* keys, const u64* d_queries, u32 n_queries, u64 n_ct, u64* d_out,
-               int partial, cudaStream_t st) {
+               int partial, cudaStream_t st, bool key_table = false) {
   if (!n_queries) return 0;
   if (n_ct != c->dim_sum / c->N + 1) {  // server.cpp:154-158
     return fail(PIRB_INVALID_ARGUMENT,
@@ -685,7 +696,7 @@ int run_answer(pirb_ctx* c, const pirb_keys* keys, const u64* d_queries, u32 n_q
   if (!pl) return rc;
   c->launches = 0;
   if (c->profiling) cudaEventRecord(c->ev[0], st);
-  RC(run_expand(c, keys, pl, d_queries, (int)n_queries, st));
+  RC(run_expand(c, keys, pl, d_queries, (int)n_queries, st, 0, -1, 0, -1, key_table));
   u64 sv_items = 0;
   for (size_t t = 0; t < pl->items.size(); ++t) sv_items = std::max(sv_items, pl->base[t] + pl->items[t]);
   RC(run_multiply(c, c->work.p, 2 * pl->cap * c->ctL, (int)n_queries, d_out, partial, st, false, (u64)pl->t_first * c->N,
@@ -745,13 +756,22 @@ int run_graphed(pirb_ctx* c, const std::tuple<int, u32, unsigned long long, cons
   return 0;
 }
 
-// Answer n_queries queries held at d_in (device-accessible) into d_out (device-accessible).
-int answer_buffers(pirb_ctx* c, const pirb_keys* keys, u32 n_queries, u64 n_ct, int partial, cudaStream_t st,
-                   const u64* d_in = nullptr, u64* d_out = nullptr) {
+// Answer n_queries queries held at d_in (device-accessible) into d_out (device-accessible).  tab: per-query Galois keys
+// (multi_key_table; `keys` is unused), uploaded into c->ktab on st here: after the caller's DevCallOrder wait, so that
+// no earlier call still reads the table, and outside any capture.  The source is pageable, so the copy has taken it
+// when cudaMemcpyAsync returns.  These calls have graphs of their own (op 3) that are not keyed on any handle.
+int answer_buffers(pirb_ctx* c, const pirb_keys* keys, const std::vector<const u64*>* tab, u32 n_queries, u64 n_ct,
+                   int partial, cudaStream_t st, const u64* d_in = nullptr, u64* d_out = nullptr) {
   if (!d_in) d_in = c->qbuf.p;
   if (!d_out) d_out = c->rbuf.p;
-  return run_graphed(c, std::make_tuple(partial, n_queries, keys ? keys->id : 0ull, (const void*)d_in, (const void*)d_out), st,
-                     [&](cudaStream_t s_) { return run_answer(c, keys, d_in, n_queries, n_ct, d_out, partial, s_); });
+  if (tab) {
+    RC(c->ktab.ensure(std::max<size_t>(tab->size() * sizeof(const u64*), 256)));
+    if (!tab->empty()) CU(cudaMemcpyAsync(c->ktab.p, tab->data(), tab->size() * sizeof(const u64*), cudaMemcpyHostToDevice, st));
+  }
+  const int op = tab ? 3 : partial;
+  const unsigned long long key_id = (!tab && keys) ? keys->id : 0ull;
+  return run_graphed(c, std::make_tuple(op, n_queries, key_id, (const void*)d_in, (const void*)d_out), st,
+                     [&](cudaStream_t s_) { return run_answer(c, keys, d_in, n_queries, n_ct, d_out, partial, s_, tab != nullptr); });
 }
 
 // All *_dev entry points work on the context's single set of workspaces, whatever stream the caller passes: each call
@@ -1209,6 +1229,7 @@ int pirb_substitute(pirb_ctx* c, const pirb_keys* keys, uint64_t* ct, uint32_t p
   L.n_queries = 1;
   L.dbg = nullptr;
   L.dbg_clock = 0;
+  L.key_tab = nullptr;
   L.xch = nullptr;
   if (c->use_cluster) {
     RC(c->xch.ensure((size_t)2 * c->N * sizeof(u64)));
@@ -1305,12 +1326,12 @@ int pirb_db_multiply(pirb_ctx* c, uint64_t* sv, uint64_t n_sv, uint64_t* out, ui
   return 0;
 }
 
-int pirb_answer(pirb_ctx* c, const pirb_keys* keys, const uint64_t* queries, uint32_t n_queries, uint64_t n_ct,
-                uint64_t* replies) {
-  if (!c || !queries || !replies) return fail(PIRB_INVALID_ARGUMENT, "null argument");
-  CU(cudaSetDevice(c->device));
-  if (c->prm.shard_count != 1) return fail(PIRB_INVALID_ARGUMENT, "pirb_answer needs an unsharded context");
+// pirb_answer and pirb_answer_multi on host buffers (tab: see answer_buffers)
+static int answer_host_common(pirb_ctx* c, const pirb_keys* keys, const std::vector<const u64*>* tab,
+                              const uint64_t* queries, uint32_t n_queries, uint64_t n_ct, uint64_t* replies) {
   cudaStream_t st = c->stream;
+  std::optional<DevCallOrder> order;  // the key table must not change under a *_dev call still in flight
+  if (tab) order.emplace(c, st);
   const size_t qbytes = (size_t)n_queries * n_ct * c->ctL * sizeof(u64);
   const size_t rbytes = (size_t)n_queries * c->reply_cts * c->ctL * sizeof(u64);
   const char* zc = getenv("PIRB_ZERO_COPY");  // read per call so that a caller can compare both paths in one process
@@ -1322,10 +1343,18 @@ int pirb_answer(pirb_ctx* c, const pirb_keys* keys, const uint64_t* queries, uin
     CU(cudaMemcpyAsync(c->qbuf.p, queries, qbytes, cudaMemcpyHostToDevice, st));
   }
   if (!r_direct) RC(c->rbuf.ensure(std::max<size_t>(rbytes, 256)));
-  RC(answer_buffers(c, keys, n_queries, n_ct, 0, st, q_direct ? U(queries) : nullptr, r_direct ? U(replies) : nullptr));
+  RC(answer_buffers(c, keys, tab, n_queries, n_ct, 0, st, q_direct ? U(queries) : nullptr, r_direct ? U(replies) : nullptr));
   if (!r_direct) CU(cudaMemcpyAsync(replies, c->rbuf.p, rbytes, cudaMemcpyDeviceToHost, st));
   CU(cudaStreamSynchronize(st));
   return 0;
+}
+
+int pirb_answer(pirb_ctx* c, const pirb_keys* keys, const uint64_t* queries, uint32_t n_queries, uint64_t n_ct,
+                uint64_t* replies) {
+  if (!c || !queries || !replies) return fail(PIRB_INVALID_ARGUMENT, "null argument");
+  CU(cudaSetDevice(c->device));
+  if (c->prm.shard_count != 1) return fail(PIRB_INVALID_ARGUMENT, "pirb_answer needs an unsharded context");
+  return answer_host_common(c, keys, nullptr, queries, n_queries, n_ct, replies);
 }
 
 // ---- ciphertext-multiplication mode (PIRParameters.use_ciphertext_multiplication; database.cpp:202-211) ----
@@ -1395,8 +1424,8 @@ int pirb_answer_ct(pirb_ctx* c, const pirb_keys* keys, const pirb_keys* relin, c
   return 0;
 }
 
-static int answer_dev_common(pirb_ctx* c, const pirb_keys* keys, const u64* d_queries, u32 n_queries, u64 n_ct,
-                             u64* d_out, int partial, cudaStream_t st) {
+static int answer_dev_common(pirb_ctx* c, const pirb_keys* keys, const std::vector<const u64*>* tab,
+                             const u64* d_queries, u32 n_queries, u64 n_ct, u64* d_out, int partial, cudaStream_t st) {
   if (!n_queries) return 0;
   if (n_ct != c->dim_sum / c->N + 1)
     return fail(PIRB_INVALID_ARGUMENT, "Number of ciphertexts doesn't match number of items for oblivious expansion.");
@@ -1407,7 +1436,7 @@ static int answer_dev_common(pirb_ctx* c, const pirb_keys* keys, const u64* d_qu
   DevCallOrder order(c, st);
   // the captured graph works on the context's own buffers; the caller's tensors are copied in and out
   CU(cudaMemcpyAsync(c->qbuf.p, d_queries, qbytes, cudaMemcpyDeviceToDevice, st));
-  RC(answer_buffers(c, keys, n_queries, n_ct, partial, st));
+  RC(answer_buffers(c, keys, tab, n_queries, n_ct, partial, st));
   CU(cudaMemcpyAsync(d_out, c->rbuf.p, rbytes, cudaMemcpyDeviceToDevice, st));
   return 0;
 }
@@ -1417,14 +1446,67 @@ int pirb_answer_dev(pirb_ctx* c, const pirb_keys* keys, const uint64_t* d_querie
   if (!c || !d_queries || !d_replies) return fail(PIRB_INVALID_ARGUMENT, "null argument");
   CU(cudaSetDevice(c->device));
   if (c->prm.shard_count != 1) return fail(PIRB_INVALID_ARGUMENT, "use pirb_answer_partial_dev on a sharded context");
-  return answer_dev_common(c, keys, U(d_queries), n_queries, n_ct, U(d_replies), 0, stream ? (cudaStream_t)stream : c->stream);
+  return answer_dev_common(c, keys, nullptr, U(d_queries), n_queries, n_ct, U(d_replies), 0,
+                           stream ? (cudaStream_t)stream : c->stream);
+}
+
+// Checks of pirb_answer_multi*, all before anything is staged, uploaded or launched, and the key table they pass on:
+// tab[j * n_queries + q] = query q's key of tree level j (Galois element N/2^j + 1).
+static int multi_key_table(pirb_ctx* c, const pirb_keys* const* keys, uint32_t n_queries, uint64_t n_ct,
+                           std::vector<const u64*>* tab) {
+  if (c->prm.shard_count != 1) return fail(PIRB_INVALID_ARGUMENT, "pirb_answer_multi needs an unsharded context");
+  if (c->ct.on) return fail(PIRB_INVALID_ARGUMENT, "pirb_answer_multi needs a re-encoder context");
+  if (!n_queries) return 0;
+  if (n_ct != c->dim_sum / c->N + 1)
+    return fail(PIRB_INVALID_ARGUMENT, "Number of ciphertexts doesn't match number of items for oblivious expansion.");
+  if (c->loaded != c->pt_count) return fail(PIRB_INVALID_ARGUMENT, "database size mismatch");
+  int rc;
+  ExpandPlan* pl = get_plan(c, c->dim_sum, 0, &rc);
+  if (!pl) return rc;
+  const u64 key_limbs = pirb_key_limbs(c);
+  tab->assign((size_t)pl->max_logm * n_queries, nullptr);
+  for (u32 q = 0; q < n_queries; ++q) {
+    const pirb_keys* kz = keys[q];
+    const std::string where = " (query " + std::to_string(q) + ")";
+    if (!kz) return fail(PIRB_INVALID_ARGUMENT, "null Galois key handle" + where);
+    if (kz->key_limbs != key_limbs || kz->device != c->device)
+      return fail(PIRB_INVALID_ARGUMENT, "Galois keys were loaded for a context of another shape" + where);
+    for (int j = 0; j < pl->max_logm; ++j) {
+      const u32 g = (c->N >> j) + 1;
+      const u64* key = kz->find(g);
+      if (!key) return fail(PIRB_INTERNAL, "Galois key not present for element " + std::to_string(g) + where);
+      (*tab)[(size_t)j * n_queries + q] = key;
+    }
+  }
+  return 0;
+}
+
+int pirb_answer_multi(pirb_ctx* c, const pirb_keys* const* keys, const uint64_t* queries, uint32_t n_queries,
+                      uint64_t n_ct, uint64_t* replies) {
+  if (!c || !keys || !queries || !replies) return fail(PIRB_INVALID_ARGUMENT, "null argument");
+  CU(cudaSetDevice(c->device));
+  std::vector<const u64*> tab;
+  RC(multi_key_table(c, keys, n_queries, n_ct, &tab));
+  if (!n_queries) return 0;
+  return answer_host_common(c, nullptr, &tab, queries, n_queries, n_ct, replies);
+}
+
+int pirb_answer_multi_dev(pirb_ctx* c, const pirb_keys* const* keys, const uint64_t* d_queries, uint32_t n_queries,
+                          uint64_t n_ct, uint64_t* d_replies, void* stream) {
+  if (!c || !keys || !d_queries || !d_replies) return fail(PIRB_INVALID_ARGUMENT, "null argument");
+  CU(cudaSetDevice(c->device));
+  std::vector<const u64*> tab;
+  RC(multi_key_table(c, keys, n_queries, n_ct, &tab));
+  return answer_dev_common(c, nullptr, &tab, U(d_queries), n_queries, n_ct, U(d_replies), 0,
+                           stream ? (cudaStream_t)stream : c->stream);
 }
 
 int pirb_answer_partial_dev(pirb_ctx* c, const pirb_keys* keys, const uint64_t* d_queries, uint32_t n_queries,
                             uint64_t n_ct, uint64_t* d_partial, void* stream) {
   if (!c || !d_queries || !d_partial) return fail(PIRB_INVALID_ARGUMENT, "null argument");
   CU(cudaSetDevice(c->device));
-  return answer_dev_common(c, keys, U(d_queries), n_queries, n_ct, U(d_partial), 1, stream ? (cudaStream_t)stream : c->stream);
+  return answer_dev_common(c, keys, nullptr, U(d_queries), n_queries, n_ct, U(d_partial), 1,
+                           stream ? (cudaStream_t)stream : c->stream);
 }
 
 int pirb_expand_ntt_dev(pirb_ctx* c, const pirb_keys* keys, const uint64_t* d_queries, uint32_t n_queries,

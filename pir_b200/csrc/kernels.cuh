@@ -19,6 +19,10 @@ struct LevelArgs {
   u32 g;         // the Galois element itself
   u64 q_stride;  // limbs between consecutive queries' workspaces
   int n_queries;
+  // per-query Galois keys (queries of different clients in one launch): device array of n_queries key pointers of
+  // this level, entry qi for query qi of the launch; nullptr: every node uses the launch's `key` argument.  Complete
+  // before the call's first kernel starts (the cluster kernels read it before griddepcontrol.wait).
+  const u64* const* key_tab;
   u64* xch;      // cluster kernel: [node][2][N] scratch through which the special-prime accumulators reach the
                  // other CTAs of the cluster (L2 moves them faster than distributed shared memory does)
   u64* dbg;      // optional per-CTA phase timestamps (clock64), 8 slots per CTA; nullptr in production
@@ -37,9 +41,10 @@ cudaError_t launch_db_preprocess(const DevParams& P, const u64* coeffs, u64* out
 
 // key switching, step 1: sigma_g(c1) digit J re-reduced mod m_I and forward-transformed -> dig[z][I][J][N]
 cudaError_t launch_ks_digits(const DevParams& P, const u64* work, const LevelArgs& L, u64* dig, cudaStream_t st);
-// step 2: acc[z][c][I] = INTT_I( sum_J dig[z][I][J] (.) key[J][c][I] )
+// step 2: acc[z][c][I] = INTT_I( sum_J dig[z][I][J] (.) key[J][c][I] ); with key_tab, node z uses
+// key_tab[z / nodes_per_query] instead of key
 cudaError_t launch_ks_mac_intt(const DevParams& P, const u64* dig, const u64* key, u64* acc, int n_nodes,
-                               cudaStream_t st);
+                               cudaStream_t st, const u64* const* key_tab = nullptr, u32 nodes_per_query = 1);
 // step 3: mod-down by P with rounding + (mode 0) SealPIR expansion combine / (mode 1) plain substitution result
 cudaError_t launch_ks_combine(const DevParams& P, u64* work, const LevelArgs& L, const u64* acc, int mode,
                               cudaStream_t st);

@@ -39,10 +39,15 @@ __device__ __forceinline__ u64 mod_down_c(u64 a, u64 last, const DevParams& P, i
   return shoup(submod(a, r, m.q), P.inv_P[j], P.inv_P_s[j], m.q);
 }
 
+// The key of the node's query: the launch's key, or with a per-query key table that query's client's key.  The first
+// generation reads it where it is used (a register holding it across the phases costs spills in <12,2,*>); the second
+// keeps it in a register (fewer spills there).
+#define PIRB_QKEY \
+  (L.key_tab ? reinterpret_cast<const u64*>(__ldg(reinterpret_cast<const unsigned long long*>(L.key_tab) + qi)) : key_arg)
 template <int LOGN, int ENG, int MODE>
 __global__ void __launch_bounds__(CCfg<LOGN>::NT, (LOGN <= 12 ? 2 : 1))
 k_ks_level_cluster(const __grid_constant__ DevParams P, u64* __restrict__ work, const LevelArgs L,
-                   const u64* __restrict__ key, int mode) {
+                   const u64* __restrict__ key_arg, int mode) {
   constexpr int N = CCfg<LOGN>::N, NT = CCfg<LOGN>::NT;
   extern __shared__ u64 smem[];
   cg::cluster_group cluster = cg::this_cluster();
@@ -90,7 +95,7 @@ k_ks_level_cluster(const __grid_constant__ DevParams P, u64* __restrict__ work, 
   {
     constexpr int LINES = N * 8 / 128;  // lines per polynomial
     for (int J = 0; J < k; ++J) {
-      const char* kp = reinterpret_cast<const char*>(key + ((u64)(J * 2 + c) * (k + 1) + I) * N);
+      const char* kp = reinterpret_cast<const char*>(PIRB_QKEY + ((u64)(J * 2 + c) * (k + 1) + I) * N);
       for (int l = tid; l < LINES; l += NT) asm volatile("prefetch.global.L2 [%0];" ::"l"(kp + (size_t)l * 128));
     }
     // Programmatic dependent launch: everything above (key prefetch, index math) may overlap the tail of the previous
@@ -171,7 +176,7 @@ k_ks_level_cluster(const __grid_constant__ DevParams P, u64* __restrict__ work, 
 #pragma unroll 2
         for (int J = 0; J < k; ++J) {
           const u64* buf = (((J & 1) == c) ? smem : peer) + (size_t)(J >> 1) * N;
-          const u64* kp = key + ((u64)(J * 2 + c) * (k + 1) + I) * N + i0;
+          const u64* kp = PIRB_QKEY + ((u64)(J * 2 + c) * (k + 1) + I) * N + i0;
           u64 dv[CH], kv[CH];
 #pragma unroll
           for (int e = 0; e < CH; ++e) {
@@ -198,7 +203,7 @@ k_ks_level_cluster(const __grid_constant__ DevParams P, u64* __restrict__ work, 
 #pragma unroll 1
         for (int J = 0; J < k; ++J) {
           const u64* buf = (((J & 1) == c) ? smem : peer) + (size_t)(J >> 1) * N;
-          const u64* kp = key + ((u64)(J * 2 + c) * (k + 1) + I) * N + i0;
+          const u64* kp = PIRB_QKEY + ((u64)(J * 2 + c) * (k + 1) + I) * N + i0;
           u64 dv[CH], kv[CH];
 #pragma unroll
           for (int e = 0; e < CH; ++e) {
@@ -320,7 +325,7 @@ k_ks_level_cluster(const __grid_constant__ DevParams P, u64* __restrict__ work, 
 template <int LOGN, int K>
 __global__ void __launch_bounds__(CCfg<LOGN>::NT, 2)
 k_ks_level_cluster2(const __grid_constant__ DevParams P, u64* __restrict__ work, const LevelArgs L,
-                    const u64* __restrict__ key, int mode) {
+                    const u64* __restrict__ key_arg, int mode) {
   constexpr int N = CCfg<LOGN>::N, NT = CCfg<LOGN>::NT;
   constexpr int NB = K < 2 ? 2 : K;  // buffers: the k digits; two accumulators live in the first two afterwards
   extern __shared__ u64 smem[];
@@ -332,6 +337,7 @@ k_ks_level_cluster2(const __grid_constant__ DevParams P, u64* __restrict__ work,
   const u32 kk = z & ((1u << L.j) - 1);
   const u32 tq = z >> L.j;
   const u32 ti = tq % L.n_trees, qi = tq / L.n_trees;
+  const u64* __restrict__ key = L.key_tab ? L.key_tab[qi] : key_arg;  // this query's client
   const u64 ctL = (u64)2 * k * N;
   const u64* src = work + qi * L.q_stride + L.src_off[ti] + kk * ctL;
   const ModC& mI = P.m[I];

@@ -125,13 +125,14 @@ k_ks_digits(const __grid_constant__ DevParams P, const u64* __restrict__ work, c
 // grid (z = node, I, c = key component)
 template <int LOGN, int ENG>
 __global__ void __launch_bounds__(Cfg<LOGN>::NT, Cfg<LOGN>::MINB)
-k_ks_mac_intt(const __grid_constant__ DevParams P, const u64* __restrict__ dig, const u64* __restrict__ key,
-              u64* __restrict__ acc) {
+k_ks_mac_intt(const __grid_constant__ DevParams P, const u64* __restrict__ dig, const u64* __restrict__ key_arg,
+              u64* __restrict__ acc, const u64* const* __restrict__ key_tab, u32 nodes_per_query) {
   constexpr int N = Cfg<LOGN>::N, NT = Cfg<LOGN>::NT;
   extern __shared__ u64 s[];
   const int tid = threadIdx.x;
   const int I = blockIdx.y, c = blockIdx.z;
   const u32 z = blockIdx.x;
+  const u64* __restrict__ key = key_tab ? key_tab[z / nodes_per_query] : key_arg;
   const int k = P.k;
   const ModC& mI = P.m[I];
   const u64* d = dig + ((u64)z * (k + 1) + I) * k * N;
@@ -464,7 +465,7 @@ cudaError_t launch_ks_digits(const DevParams& P, const u64* work, const LevelArg
 }
 
 cudaError_t launch_ks_mac_intt(const DevParams& P, const u64* dig, const u64* key, u64* acc, int n_nodes,
-                               cudaStream_t st) {
+                               cudaStream_t st, const u64* const* key_tab, u32 nodes_per_query) {
   if (n_nodes <= 0) return cudaSuccess;
   return dispatch(P, [&](auto ln, auto lz) {
     constexpr int LN = decltype(ln)::value;
@@ -472,7 +473,7 @@ cudaError_t launch_ks_mac_intt(const DevParams& P, const u64* dig, const u64* ke
     auto kern = k_ks_mac_intt<LN, LZ>;
     cudaError_t e = ensure_smem(kern, Cfg<LN>::SMEM);
     if (e != cudaSuccess) return e;
-    kern<<<dim3(n_nodes, P.k + 1, 2), Cfg<LN>::NT, Cfg<LN>::SMEM, st>>>(P, dig, key, acc);
+    kern<<<dim3(n_nodes, P.k + 1, 2), Cfg<LN>::NT, Cfg<LN>::SMEM, st>>>(P, dig, key, acc, key_tab, nodes_per_query);
     return cudaGetLastError();
   });
 }
